@@ -24,6 +24,10 @@ CUDA events around its launches (gsicp_prof_*); `cpu_baseline` = the reference's
 /root/reference into oracle/_ref) + the CPU raster oracle on a bounded sample.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c3|c2|c4|c5] [--multi replicas|shard]
+                  [--dump-outputs DIR]
+`--dump-outputs DIR` writes what the headline run's last timed frame returned to its caller (pose, correspondences, rendered
+images, radii, loss, the map's gradients) as DIR/<name>.npy, so that two builds can be compared output for output: the
+inputs are seeded, so the same arguments give the same inputs.
 `--impl reference` = the reference's own implementation of the same frame on this box: fast_gicp (its unmodified
 sources + pybind module, oracle/_ref/fast_gicp) on all host cores in a tracker process + the reference's CUDA
 rasterizer through its own torch extension (oracle/_ref/site, stock build path) and PyTorch loss in the mapper process.
@@ -73,6 +77,8 @@ def parse():
                     help="N>1 with c3/c2: replicas = one independent SLAM sequence per GPU, no collective (the SLAM loop is "
                          "sequential in time: SURVEY §8e 'replicas only'); shard = ONE sequence, raster tiles + GICP source "
                          "points sharded over the ranks (pays only at C4/C5 sizes)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the headline run's last timed step as DIR/<name>.npy (float32 / float64)")
     ap.add_argument("--loss", default="torch", choices=["torch", "fused", "l1"],
                     help="mapper loss of the HEADLINE leg.  torch (default) = the reference's PyTorch ops (what an unmodified "
                          "mp_Mapper.py runs, and what the reference arm runs); fused = gs_icp_slam_b200.loss.mapping_loss; "
@@ -258,6 +264,7 @@ class Ours:
         self.pose = frames[0]["c2w"].astype(np.float32)
         self.pool = None
         self.gicp_stream = None
+        self.keep = None  # dict: the outputs of the latest step are kept here (--dump-outputs)
         self.stats = dict(R=0, V=0, n_src=0, n_corr=0, n_tgt=0, frames=0, h2d=0, d2h=0, n_lin=0, pose_err=0.0)
         self.refresh_target(resident=True)
 
@@ -296,6 +303,8 @@ class Ours:
         st["n_lin"] += self.reg.last_iterations
         st["pose_err"] = max(st["pose_err"], float(np.abs(pose.astype(np.float64) - f["c2w"]).max()))
         self.pose = pose
+        if self.keep is not None:
+            self.keep.update(pose=pose, correspondences=corr, sq_distances=sqd)
         if (step + 1) % KEYFRAME_EVERY == 0:
             rots, scales = self.reg.get_source_rotationsq(), self.reg.get_source_scales()
             st["d2h"] += rots.nbytes + scales.nbytes
@@ -332,6 +341,9 @@ class Ours:
         loss.backward()
         lv = float(loss.item())  # D2H read of the step's result
         st["d2h"] += 8
+        if self.keep is not None:  # references only: the copies are made after the timed steps
+            self.keep.update(loss=lv, color=color, depth=depth, radii=radii, grad_means2D=self.means2D.grad,
+                             **{"grad_" + k: m[k].grad for k in m})
         for k in m:
             m[k].grad = None
         self.means2D.grad = None
@@ -640,6 +652,37 @@ def ncu_traffic():
         return {}
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(out_dir, kept, rank, world, n_gaussians):
+    """Writes the kept outputs of one step as float32 / float64 .npy files (integer outputs become float64, exactly); with
+    several ranks each writes its own subdirectory rank<N>/.  Above DUMP_LIMIT bytes in all, the per-Gaussian arrays keep a
+    fixed, seeded sample of Gaussians, whose indices are written as gaussian_index.npy."""
+    import torch
+
+    if world > 1:
+        out_dir = os.path.join(out_dir, f"rank{rank}")
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {}
+    for name, v in kept.items():
+        if v is None:
+            continue
+        a = v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)
+        arrays[name] = a.astype(np.float64 if a.dtype.kind in "biu" or a.dtype == np.float64 or a.ndim == 0 else np.float32)
+    per_gaussian = [k for k, a in arrays.items() if a.ndim >= 1 and a.shape[0] == n_gaussians]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        row = sum(arrays[k].nbytes for k in per_gaussian) / n_gaussians
+        keep = int((DUMP_LIMIT - (total - row * n_gaussians)) // (row + 8))
+        idx = np.sort(np.random.default_rng(0).choice(n_gaussians, keep, replace=False))
+        for k in per_gaussian:
+            arrays[k] = arrays[k][idx]
+        arrays["gaussian_index"] = idx.astype(np.float64)
+    for name, a in sorted(arrays.items()):
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def bind_to_gpu_numa(local_rank, world):
     """N > 1 on one host: pin this rank (its Python threads, the library's spin-waits, pinned-staging copies) to the CPUs
     of its GPU's NUMA node, split evenly among the ranks that share the node (r1: e2e replica efficiency 0.71 at N = 8 with
@@ -675,6 +718,8 @@ def main():
     rank = int(os.environ.get("RANK", 0))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
+    if args.dump_outputs and (args.config in ("c1", "c4", "c5") or args.impl != "ours"):
+        raise SystemExit("bench.py: --dump-outputs writes the SLAM frame of --impl ours (configs c3, c2)")
     if args.config in ("c1", "c4", "c5"):
         from tools import bench_large
 
@@ -727,8 +772,12 @@ def main():
         eng.enable_concurrent(concurrent)
         if concurrent:
             eng.run(pre, 1, resident=True)  # stream / thread start-up, untimed
+        eng.keep = {} if args.dump_outputs else None
         r = eng.run(K, Wm, resident=True)
         res_times = list(eng.last_times)
+        if eng.keep is not None:
+            dump_outputs(args.dump_outputs, eng.keep, rank, world, args.gaussians)
+            eng.keep = None
         e = eng.run(K, Wm, resident=False)
         e2e_times = list(eng.last_times)
     clocks = clk.summary()

@@ -1,13 +1,17 @@
 """Call sequences shared by the GICP parity tests.  Every case takes a `make()` factory returning an object with the
-pygicp.FastGICP interface (this repo's CUDA drop-in, the CPU oracle, or the reference's own pybind11 module built from
-/root/reference: oracle/ref_gicp.py) and returns a dict of numpy results to compare."""
+pygicp.FastGICP interface (this repo's CUDA drop-in, the CPU oracle, or the reference's own pybind11 module:
+oracle/ref_gicp.py) and returns a dict of numpy results to compare.  The reference's results are stored in
+tests/golden/gicp_fastgicp_cases.npz (tests/golden/make_gicp_ref_cases.py)."""
 import os
 
 import numpy as np
 
 from gs_icp_slam_b200 import synthetic as S
+from tests.refdigest import Golden, record
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+REF_CASES = os.path.join(HERE, "golden", "gicp_fastgicp_cases.npz")
+EXACT = ("corr", "sqd", "tgt_rots", "src_rots", "tgt_scales", "src_scales", "rots_kf", "scales_kf")
 
 
 def _params(r, max_corr):
@@ -84,8 +88,7 @@ def kitti(make):
     return out
 
 
-def compare(a, b, exact_prefixes=("corr", "sqd", "tgt_rots", "src_rots", "tgt_scales", "src_scales", "rots_kf", "scales_kf"),
-            pose_tol=1e-6, h_rtol=1e-9):
+def compare(a, b, exact_prefixes=EXACT, pose_tol=1e-6, h_rtol=1e-9):
     """Parity bars (BASELINE.json north_star): indices / squared distances / float32 exports bit-exact, pose SE(3)
     within 1e-6, fp64 normal equations within h_rtol of their largest entry."""
     for k in a:
@@ -153,3 +156,33 @@ def duplicates_and_outliers(make):
     out.update(corr=np.array(c), sqd=np.array(d), tgt_rots=np.array(r.get_target_rotationsq()), tgt_scales=np.array(r.get_target_scales()),
                src_rots=np.array(r.get_source_rotationsq()), src_scales=np.array(r.get_source_scales()), H=np.array(r.get_final_hessian()))
     return out
+
+
+def store(out, case, res):
+    """Adds a case's results to the dict `out`: the bit-exact outputs as records (tests/refdigest.py), the rest in full."""
+    for k, v in res.items():
+        v = np.asarray(v)
+        if k.startswith(EXACT):
+            record(out, f"{case}/{k}", v, sample=False)
+        else:
+            out[f"{case}/{k}"] = v
+
+
+def stored(case, gold=None):
+    """(the fully stored results of `case`, the Golden reader) from tests/golden/gicp_fastgicp_cases.npz."""
+    gold = gold or Golden(REF_CASES)
+    pre = case + "/"
+    return {k[len(pre):]: v for k, v in gold.z.items() if k.startswith(pre) and "." not in k[len(pre):]}, gold
+
+
+def compare_stored(a, case, gold=None, **kw):
+    """compare(a, reference results of `case`): bit-exact outputs through their records, dtype included."""
+    full, gold = stored(case, gold)
+    compare({k: a[k] for k in a if k in full}, full, **kw)
+    for k in a:
+        if k in full or k in ("T_gt", "relative", "gt_last"):
+            continue
+        assert k.startswith(kw.get("exact_prefixes", EXACT)), f"unclassified key {k}"
+        x = np.asarray(a[k])
+        assert x.dtype.str == str(gold.z[f"{case}/{k}.dtype"]) and gold.equal(f"{case}/{k}", x), k
+    return full, gold

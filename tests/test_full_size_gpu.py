@@ -1,11 +1,12 @@
-"""BASELINE.json's full sizes, through properties that do not need an oracle run of the same size plus — where the
-reference CUDA build is present — a direct comparison:
+"""BASELINE.json's full sizes, through properties that do not need an oracle run of the same size plus a direct comparison
+with records of the reference's own CUDA code at the same sizes (tests/golden/raster_ref_records.npz):
   C3 640x480 / 300k Gaussians and C4 1280x960 / 1M Gaussians (rasterizer), C5-shape 2M x 2M points (GICP)."""
 import numpy as np
 import pytest
 import torch
 
 from gs_icp_slam_b200 import synthetic as S
+from tests.refdigest import RASTER_RECORDS, Golden
 from tests.util import rel_err, scene_tensors
 
 pytestmark = pytest.mark.gpu
@@ -28,7 +29,6 @@ def _bw(R, t, c, bg, out, gdep, gcol):
 @pytest.mark.parametrize("P,size,scale", [(300000, (640, 480), 1.0), (1000000, (1280, 960), 2.0)])
 def test_rasterizer_full_size_properties(cuda, P, size, scale):
     from gs_icp_slam_b200 import rasterizer as R
-    from oracle import ref_cuda
 
     g, cm, t, c, cam = scene_tensors(P, 3 if P == 300000 else 4, cuda, size=size, scale=scale)
     W, H = size
@@ -71,16 +71,13 @@ def test_rasterizer_full_size_properties(cuda, P, size, scale):
     for x in a:
         if x.numel():
             assert float(x[inv].abs().max()) == 0.0
-    if ref_cuda.available():  # the reference's own CUDA code at the same size: bit-exact lists and images
-        ref = ref_cuda.RefRaster(bg, t["means3D"], t["shs"], None, t["opacities"].reshape(-1), t["scales"], t["rotations"], None,
-                                 c["viewmatrix"], c["projmatrix"], c["campos"], c["tanfovx"], c["tanfovy"], H, W, 0)
-        rpl, rrg = ref.export()
-        assert n == ref.num_rendered and torch.equal(pl, rpl) and torch.equal(rg, rrg)
-        assert torch.equal(radii, ref.radii) and torch.equal(color, ref.color) and torch.equal(depth, ref.depth)
-        rgrad = ref.backward(g1c, g1d)
-        for name, o in zip(["means2D", "colors", "opacity", "means3D", "cov3D", "sh", "scales", "rotations"], a):
-            assert rel_err(o.cpu().numpy(), rgrad[name].cpu().numpy()) <= 2e-4, name
-        ref.free()
+    # the reference's own CUDA code at the same size: bit-exact lists and images
+    gold, k = Golden(RASTER_RECORDS), f"full_{P}/"
+    assert n == gold.scalar(k + "num_rendered") and gold.equal(k + "point_list", pl.to(torch.int64))
+    assert gold.equal(k + "ranges", rg.to(torch.int64))
+    assert gold.equal(k + "radii", radii) and gold.equal(k + "color", color) and gold.equal(k + "depth", depth)
+    for name, o in zip(["means2D", "colors", "opacity", "means3D", "cov3D", "sh", "scales", "rotations"], a):
+        assert gold.rel_err(k + "grad_" + name, o) <= 2e-4, name
 
 
 def test_gicp_full_size_recovers_the_pose(cuda):

@@ -234,12 +234,12 @@ def test_dist2_matches_bruteforce_and_reference(cuda):
     np.fill_diagonal(d, np.inf)
     ref = np.sort(d, axis=1)[:, :3].mean(1)
     assert np.allclose(out, ref, rtol=2e-5, atol=1e-12)
-    from oracle import ref_cuda
+    # against the reference's simple-knn on 200k points, through its recorded output (tests/golden/raster_ref_records.npz)
+    from tests.refdigest import RASTER_RECORDS, Golden
 
-    if ref_cuda.available():
-        big = torch.from_numpy(S.sample_surface(200000, 41, 0.002)[0].astype(np.float32)).to(cuda)
-        a, b = distCUDA2(big), ref_cuda.ref_dist2(big)
-        assert torch.allclose(a, b, rtol=2e-5, atol=1e-12)
+    big = torch.from_numpy(S.sample_surface(200000, 41, 0.002)[0].astype(np.float32)).to(cuda)
+    a, b, _ = Golden(RASTER_RECORDS).sample("dist2_200000/dist2", distCUDA2(big))
+    assert np.allclose(a, b, rtol=2e-5, atol=1e-12)
     assert torch.isinf(distCUDA2(torch.zeros((2, 3), device=cuda))).all()  # fewer than 3 neighbours -> inf, like FLT_MAX sums
 
 

@@ -1,5 +1,6 @@
 """CPU tests: the GICP oracle (oracle/gicp_oracle.cpp) against
-  * the reference's vendored Eigen (oracle/_ref/libref_gicp_eigen.so: JacobiSVD, Quaterniond, inverse, LDLT),
+  * the reference's vendored Eigen (oracle/_ref/libref_gicp_eigen.so: JacobiSVD, Quaterniond, inverse, LDLT), through its
+    outputs on these inputs stored in tests/golden/gicp_eigen_calls.npz (tests/golden/make_gicp_eigen_golden.py),
   * brute-force numpy k-NN,
   * the committed golden vectors (tests/golden/gicp_*.npz), incl. the reference's own acceptance fixture
     (KITTI pair + relative.txt, bound 0.05 m / 1 deg: submodules/fast_gicp/src/test/gicp_test.cpp:147-201)."""
@@ -14,13 +15,50 @@ from oracle import gicp_oracle as G
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 EIG = os.path.join(os.path.dirname(HERE), "oracle", "_ref", "libref_gicp_eigen.so")
+EIG_CALLS = os.path.join(HERE, "golden", "gicp_eigen_calls.npz")
+# output arguments of the libref_gicp_eigen.so functions the tests call: (argument position, dtype, element count)
+EIG_OUT = {"eig_svd3": [(1, "f8", 9), (2, "f8", 3), (3, "f8", 9)], "eig_quat_from_matrix": [(1, "f8", 4)],
+           "eig_ldlt_solve6": [(2, "f8", 6)], "eig_so3_exp": [(1, "f8", 9)],
+           "eig_cov_pipeline": [(2, "f4", 4), (3, "f4", 3), (4, "f8", 9)], "eig_cov_from_qs": [(2, "f8", 9)]}
 
 
-@pytest.fixture(scope="module")
-def eig():
-    if not os.path.exists(EIG):
-        pytest.skip("oracle/_ref/libref_gicp_eigen.so not built (needs /root/reference)")
-    return C.CDLL(EIG)
+class EigenRecorder:
+    """Calls the Eigen build and keeps the outputs of every call, in call order (tests/golden/make_gicp_eigen_golden.py)."""
+
+    def __init__(self, lib):
+        self.lib, self.calls = lib, {k: [] for k in EIG_OUT}
+
+    def __getattr__(self, name):
+        def call(*args):
+            getattr(self.lib, name)(*args)
+            self.calls[name].append([np.ctypeslib.as_array(C.cast(args[i].value, C.POINTER(C.c_double if t == "f8" else C.c_float)),
+                                                           (n,)).copy() for i, t, n in EIG_OUT[name]])
+        return call
+
+    def arrays(self, prefix):
+        return {f"{prefix}{name}.{i}": np.array([c[j] for c in calls]).reshape(len(calls), n)
+                for name, calls in self.calls.items() for j, (i, t, n) in enumerate(EIG_OUT[name])}
+
+
+class EigenReplay:
+    """Stands in for the Eigen build: each call writes the outputs the build produced for the same call of the same test."""
+
+    def __init__(self, arrays, prefix):
+        self.arrays, self.next = {k[len(prefix):]: v for k, v in arrays.items() if k.startswith(prefix)}, {k: 0 for k in EIG_OUT}
+
+    def __getattr__(self, name):
+        def call(*args):
+            k = self.next[name]
+            self.next[name] += 1
+            for i, t, n in EIG_OUT[name]:
+                a = np.ascontiguousarray(self.arrays[f"{name}.{i}"][k], dtype=t)
+                C.memmove(args[i].value, a.ctypes.data, a.nbytes)
+        return call
+
+
+@pytest.fixture()
+def eig(request):
+    return EigenReplay(dict(np.load(EIG_CALLS)), request.function.__name__ + "/")
 
 
 def _p(a):
@@ -151,7 +189,26 @@ def test_cov_from_qs_quirk_matches_eigen(eig):
         assert np.allclose(covs[i], out, rtol=1e-10, atol=1e-14)
 
 
-def test_linearize_matches_eigen_per_point(eig):
+def eigen_linearize(lib, r, pose, corr, src, tgt):
+    """Eigen's per-point Mahalanobis matrix and linearisation summed over the correspondences: (H, b, error)."""
+    s32, t32 = src.astype(np.float32), tgt.astype(np.float32)
+    ca, cb = r.get_source_covariances(), r.get_target_covariances()
+    He, be, ee = np.zeros((6, 6)), np.zeros(6), 0.0
+    for i in range(len(src)):
+        j = corr[i]
+        if j < 0:
+            continue
+        M, Hi, bi, ei = np.empty((3, 3)), np.empty((6, 6)), np.empty(6), C.c_double(0)
+        lib.eig_mahalanobis(_p(np.ascontiguousarray(ca[i])), _p(np.ascontiguousarray(cb[j])), _p(pose), _p(M))
+        lib.eig_linearize_point(_p(pose), _p(s32[i].copy()), _p(t32[j].copy()), _p(M), _p(Hi), _p(bi), C.byref(ei))
+        He += Hi
+        be += bi
+        ee += ei.value
+    return He, be, ee
+
+
+def linearize_case():
+    """The oracle's linearisation on a perturbed pose: (oracle, pose, correspondences, squared distances, source, target)."""
     tgt, src, T = S.gicp_pair(600, 400, 8, 9, 0.002)
     r = G.FastGICP()
     r.set_max_correspondence_distance(0.5)
@@ -163,6 +220,11 @@ def test_linearize_matches_eigen_per_point(eig):
     pose = np.ascontiguousarray(T + 1e-3 * np.random.default_rng(1).normal(size=(4, 4)) * np.array([[1, 1, 1, 1]] * 3 + [[0, 0, 0, 0]]))
     H, b, err = r.linearize(pose)
     corr, sqd = r.get_source_correspondence()
+    return r, pose, corr, sqd, src, tgt, (H, b, err)
+
+
+def test_linearize_matches_eigen_per_point():
+    r, pose, corr, sqd, src, tgt, (H, b, err) = linearize_case()
     # correspondences: brute force with the same fp32 transform
     Pf = pose.astype(np.float32)
     s32, t32 = src.astype(np.float32), tgt.astype(np.float32)
@@ -173,18 +235,7 @@ def test_linearize_matches_eigen_per_point(eig):
     d2 = (d[..., 0] + d[..., 1]) + d[..., 2]
     assert np.array_equal(corr, np.where(d2.min(1) < 0.25, d2.argmin(1), -1))
     assert np.array_equal(sqd, d2.min(1))
-    ca, cb = r.get_source_covariances(), r.get_target_covariances()
-    He, be, ee = np.zeros((6, 6)), np.zeros(6), 0.0
-    for i in range(len(src)):
-        j = corr[i]
-        if j < 0:
-            continue
-        M, Hi, bi, ei = np.empty((3, 3)), np.empty((6, 6)), np.empty(6), C.c_double(0)
-        eig.eig_mahalanobis(_p(np.ascontiguousarray(ca[i])), _p(np.ascontiguousarray(cb[j])), _p(pose), _p(M))
-        eig.eig_linearize_point(_p(pose), _p(s32[i].copy()), _p(t32[j].copy()), _p(M), _p(Hi), _p(bi), C.byref(ei))
-        He += Hi
-        be += bi
-        ee += ei.value
+    He, be, ee = (np.load(EIG_CALLS)[k] for k in ("linearize.H", "linearize.b", "linearize.e"))
     assert np.allclose(H, He, rtol=1e-9, atol=1e-9 * np.abs(He).max())
     assert np.allclose(b, be, rtol=1e-9, atol=1e-9 * np.abs(be).max())
     assert abs(err - ee) <= 1e-9 * abs(ee)

@@ -1,7 +1,10 @@
 """N4 (SURVEY.md §8f): scene.ply written by gs_icp_slam_b200.map_table — byte layout, round trip, and byte-for-byte equality
 with the reference's own GaussianModel.save_ply (scene/gaussian_model.py:619-636, imported unmodified from the installed copy
 under oracle/_ref/gs_icp_slam; the `plyfile` package it calls is absent from this image and replaced by oracle/stubs/plyfile.py,
-which only serialises the structured array the reference hands it)."""
+which only serialises the structured array the reference hands it).  The reference's output is stored as its size and SHA-256
+in tests/golden/scene_ply_ref.json (tests/golden/make_scene_ply_golden.py)."""
+import hashlib
+import json
 import os
 import sys
 
@@ -11,6 +14,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_SLAM = os.path.join(ROOT, "oracle", "_ref", "gs_icp_slam")
+GOLD = os.path.join(ROOT, "tests", "golden", "scene_ply_ref.json")
 
 
 def _params(n, degree, seed=0):
@@ -49,11 +53,9 @@ def test_layout_and_round_trip(tmp_path, n, degree):
         read_scene_ply(path, degree + 1)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_SLAM), reason="oracle/_ref/gs_icp_slam not installed (oracle/install_ref_slam.sh)")
-@pytest.mark.parametrize("degree", [0, 3])
-def test_same_bytes_as_reference_save_ply(tmp_path, degree):
-    from gs_icp_slam_b200.map_table import write_scene_ply
-
+def reference_save_ply(path, degree):
+    """The reference's own GaussianModel.save_ply on the seeded parameters of the byte-equality test (needs its SLAM scripts
+    installed under oracle/_ref/gs_icp_slam; used by tests/golden/make_scene_ply_golden.py)."""
     saved_path, saved_mods = list(sys.path), set(sys.modules)
     sys.path[:0] = [ROOT, os.path.join(ROOT, "oracle", "stubs"), REF_SLAM]
     try:
@@ -63,12 +65,22 @@ def test_same_bytes_as_reference_save_ply(tmp_path, degree):
         gm = GaussianModel(degree)
         gm._xyz, gm._features_dc, gm._features_rest = p["xyz"], p["features_dc"], p["features_rest"]
         gm._opacity, gm._scaling, gm._rotation = p["opacity"], p["scaling"], p["rotation"]
-        ref_path, our_path = str(tmp_path / "ref" / "scene.ply"), str(tmp_path / "ours" / "scene.ply")
-        gm.save_ply(ref_path)
-        write_scene_ply(our_path, **p)
-        assert open(ref_path, "rb").read() == open(our_path, "rb").read()
+        gm.save_ply(path)
     finally:
         sys.path[:] = saved_path
         for k in list(sys.modules):
             if k not in saved_mods and k.split(".")[0] in ("scene", "utils", "arguments", "plyfile", "open3d", "rerun", "torchmetrics"):
                 del sys.modules[k]
+
+
+@pytest.mark.parametrize("degree", [0, 3])
+def test_same_bytes_as_reference_save_ply(tmp_path, degree):
+    """Byte-for-byte equality with the file the reference's save_ply writes, through its size and SHA-256
+    (tests/golden/scene_ply_ref.json)."""
+    from gs_icp_slam_b200.map_table import write_scene_ply
+
+    ref = json.load(open(GOLD))[str(degree)]
+    our_path = str(tmp_path / "ours" / "scene.ply")
+    write_scene_ply(our_path, **_params(300, degree, seed=3))
+    blob = open(our_path, "rb").read()
+    assert len(blob) == ref["bytes"] and hashlib.sha256(blob).hexdigest() == ref["sha256"]
