@@ -136,7 +136,6 @@ _sig("gsicp_raster_set_comm", i32, [vp])
 _sig("gsicp_mapping_loss_work_bytes", C.c_size_t, [i32, i32])
 _sig("gsicp_mapping_loss_forward", i32, [i32, i32, vp, vp, vp, vp, C.c_float, C.c_float, C.c_float, i32, vp, vp, vp, vp, vp])
 _sig("gsicp_mapping_loss_backward", i32, [i32, i32, vp, vp, vp, vp, C.c_float, C.c_float, C.c_float, i32, vp, vp, vp, vp, vp])
-_sig("gsicp_gicp_last_timing", i32, [vp, vp])
 
 # BOUND lists every bound symbol; tests/test_abi.py checks include/gsicp_b200.h against it.
 

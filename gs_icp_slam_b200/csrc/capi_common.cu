@@ -21,6 +21,47 @@ void set_error(const char* fmt, ...) {
   vsnprintf(g_err, sizeof(g_err), fmt, ap);
   va_end(ap);
 }
+
+int HostMailbox::ensure(size_t bytes) {
+  if (host) return GSICP_OK;
+  GSICP_CUDA(cudaHostAlloc((void**)&host, bytes, cudaHostAllocMapped));
+  std::memset(host, 0, bytes);
+  const cudaError_t e = cudaHostGetDevicePointer((void**)&dev, host, 0);
+  if (e != cudaSuccess) {
+    release();
+    set_error("cudaHostGetDevicePointer failed: %s", cudaGetErrorString(e));
+    return GSICP_ECUDA;
+  }
+  return GSICP_OK;
+}
+
+int HostMailbox::wait(size_t word, unsigned long long s, cudaStream_t stream, const char* what) const {
+  const volatile unsigned long long* p = host + word;
+  long spins = 0;
+  while (*p != s) {
+#if defined(__x86_64__)
+    __builtin_ia32_pause();
+#endif
+    if ((++spins & 0xfffff) == 0) {
+      const cudaError_t q = cudaStreamQuery(stream);
+      if (q != cudaSuccess && q != cudaErrorNotReady) {
+        set_error("%s failed: %s", what, cudaGetErrorString(q));
+        return GSICP_ECUDA;
+      }
+      if (q == cudaSuccess && *p != s) {
+        set_error("%s was not published", what);
+        return GSICP_ECUDA;
+      }
+    }
+  }
+  std::atomic_thread_fence(std::memory_order_acquire);  // the caller's reads of the published words come after this one
+  return GSICP_OK;
+}
+
+void HostMailbox::release() {
+  if (host) cudaFreeHost(host);
+  host = dev = nullptr;
+}
 }  // namespace gsicp
 
 namespace gsicp {

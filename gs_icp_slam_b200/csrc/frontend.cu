@@ -10,9 +10,9 @@
 //                             (R p - R T with the INVERSE pose's R, T as the script forms them), q_cam (x) rots for every
 //                             point (quaternion_multiply, :385-392), and eliminate_overlapped2 (:374-380): the trackable
 //                             slots whose squared NN distance exceeds the threshold, compacted.
-#include <cub/cub.cuh>
 #include <mutex>
 #include "host_common.h"
+#include "scan.cuh"
 
 namespace gsicp {
 
@@ -153,55 +153,9 @@ keep_far_kernel(int n_trk, FarFlag f, const int* __restrict__ excl, const int32_
 struct FrontScratch {
   std::mutex mu;
   Scratch excl, cub_tmp;
-  unsigned long long* h_map = nullptr;
-  unsigned long long* d_map = nullptr;
-  unsigned long long seq = 0;
+  HostMailbox box;  // [0] point / kept count, [1] trackable count, [2] and [3] their sequence words
 };
 static FrontScratch g_front;
-
-template <typename Flag>
-static int front_scan(int n, Flag flag, cudaStream_t stream) {
-  if (int e = g_front.excl.ensure((size_t)n * sizeof(int))) return e;
-  cub::CountingInputIterator<int> counting(0);
-  cub::TransformInputIterator<int, Flag, cub::CountingInputIterator<int>> flags(counting, flag);
-  size_t tmp = 0;
-  cub::DeviceScan::ExclusiveSum(nullptr, tmp, flags, g_front.excl.as<int>(), n, stream);
-  if (int e = g_front.cub_tmp.ensure(tmp)) return e;
-  tmp = g_front.cub_tmp.cap;
-  GSICP_CUDA(cub::DeviceScan::ExclusiveSum(g_front.cub_tmp.ptr, tmp, flags, g_front.excl.as<int>(), n, stream));
-  return GSICP_OK;
-}
-
-static int front_map() {
-  if (!g_front.h_map) {
-    GSICP_CUDA(cudaHostAlloc((void**)&g_front.h_map, 4 * sizeof(unsigned long long), cudaHostAllocMapped));
-    for (int i = 0; i < 4; i++) g_front.h_map[i] = 0;
-    GSICP_CUDA(cudaHostGetDevicePointer((void**)&g_front.d_map, g_front.h_map, 0));
-  }
-  return GSICP_OK;
-}
-
-static int front_wait(int word, unsigned long long seq, cudaStream_t stream) {
-  volatile unsigned long long* pm = g_front.h_map;
-  long spins = 0;
-  while (pm[word] != seq) {
-#if defined(__x86_64__)
-    __builtin_ia32_pause();
-#endif
-    if ((++spins & 0xfffff) == 0) {
-      const cudaError_t q = cudaStreamQuery(stream);
-      if (q != cudaSuccess && q != cudaErrorNotReady) {
-        set_error("front-end kernel failed: %s", cudaGetErrorString(q));
-        return GSICP_ECUDA;
-      }
-      if (q == cudaSuccess && pm[word] != seq) {
-        set_error("front-end count was not published");
-        return GSICP_ECUDA;
-      }
-    }
-  }
-  return GSICP_OK;
-}
 
 }  // namespace gsicp
 
@@ -223,28 +177,29 @@ extern "C" int gsicp_frontend_cloud(const uint16_t* d_depth, const uint8_t* d_rg
   }
   cudaStream_t stream = (cudaStream_t)stream_v;
   std::lock_guard<std::mutex> lock(g_front.mu);
-  if (int e = front_map()) return e;
+  HostMailbox& box = g_front.box;
+  if (int e = box.ensure(4 * sizeof(unsigned long long))) return e;
   CloudArgs a;
   a.W = W; a.H = H; a.step = step; a.rows = H / step + 1; a.cols = (W + step - 1) / step;
   a.fx = fx; a.fy = fy; a.cx = cx; a.cy = cy; a.depth_scale = depth_scale; a.depth_trunc = depth_trunc;
   a.depth = d_depth; a.rgb = d_rgb;
   const int ns = a.rows * a.cols;
-  if (int e = front_scan(ns, NonZeroDepth{a}, stream)) return e;
-  const unsigned long long seq = ++g_front.seq;
+  if (int e = flag_exclusive_scan<int>(ns, NonZeroDepth{a}, g_front.excl, g_front.cub_tmp, stream)) return e;
+  const unsigned long long seq = ++box.seq;
   GSICP_LAUNCH(cloud_kernel, (ns + 255) / 256, 256, 0, stream, a, ns, g_front.excl.as<int>(), d_points, d_colors, d_z, d_filter,
                (unsigned int*)nullptr);
-  GSICP_LAUNCH(publish_count_kernel, 1, 1, 0, stream, ns, g_front.excl.as<int>(), a, g_front.d_map, seq);
+  GSICP_LAUNCH(publish_count_kernel, 1, 1, 0, stream, ns, g_front.excl.as<int>(), a, box.dev, seq);
   GSICP_CUDA(cudaGetLastError());
-  if (int e = front_wait(2, seq, stream)) return e;
-  const int n = (int)g_front.h_map[0];
+  if (int e = box.wait(2, seq, stream, "front-end point count")) return e;
+  const int n = (int)box.host[0];
   *n_points = n;
   *n_trackable = 0;
   if (n == 0) return GSICP_OK;
-  if (int e = front_scan(n, FlagAt{d_filter}, stream)) return e;
-  GSICP_LAUNCH(slots_kernel, (n + 255) / 256, 256, 0, stream, n, g_front.excl.as<int>(), d_filter, d_trackable, g_front.d_map, seq, 1);
+  if (int e = flag_exclusive_scan<int>(n, FlagAt{d_filter}, g_front.excl, g_front.cub_tmp, stream)) return e;
+  GSICP_LAUNCH(slots_kernel, (n + 255) / 256, 256, 0, stream, n, g_front.excl.as<int>(), d_filter, d_trackable, box.dev, seq, 1);
   GSICP_CUDA(cudaGetLastError());
-  if (int e = front_wait(3, seq, stream)) return e;
-  *n_trackable = (int)g_front.h_map[1];
+  if (int e = box.wait(3, seq, stream, "front-end trackable count")) return e;
+  *n_trackable = (int)box.host[1];
   return GSICP_OK;
 }
 
@@ -275,14 +230,15 @@ extern "C" int gsicp_frontend_not_overlapped(int n_trackable, const float* d_sq_
   if (n_trackable == 0) return GSICP_OK;
   cudaStream_t stream = (cudaStream_t)stream_v;
   std::lock_guard<std::mutex> lock(g_front.mu);
-  if (int e = front_map()) return e;
+  HostMailbox& box = g_front.box;
+  if (int e = box.ensure(4 * sizeof(unsigned long long))) return e;
   const FarFlag f{d_sq_dist, threshold};
-  if (int e = front_scan(n_trackable, f, stream)) return e;
-  const unsigned long long seq = ++g_front.seq;
+  if (int e = flag_exclusive_scan<int>(n_trackable, f, g_front.excl, g_front.cub_tmp, stream)) return e;
+  const unsigned long long seq = ++box.seq;
   GSICP_LAUNCH(keep_far_kernel, (n_trackable + 255) / 256, 256, 0, stream, n_trackable, f, g_front.excl.as<int>(), d_trackable, d_out,
-               g_front.d_map, seq);
+               box.dev, seq);
   GSICP_CUDA(cudaGetLastError());
-  if (int e = front_wait(2, seq, stream)) return e;
-  *n_out = (int)g_front.h_map[0];
+  if (int e = box.wait(2, seq, stream, "front-end kept count")) return e;
+  *n_out = (int)box.host[0];
   return GSICP_OK;
 }

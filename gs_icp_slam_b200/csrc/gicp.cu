@@ -23,9 +23,6 @@
 #include <vector>
 #include "gicp_math.cuh"
 #include <algorithm>
-#include <atomic>
-#include <thread>
-#include <vector>
 
 #include "grid.cuh"
 #include "comm.cuh"
@@ -232,9 +229,9 @@ __device__ __forceinline__ double warp_sum_d(double v) {
 // block-level reduction of NV doubles per thread into partial[blockIdx][NV]; the last block to finish
 // sums the partials in block order (deterministic) into out[NV].
 //
-// When `host_out` is non-null (single-GPU runs) the last block also publishes the sums into MAPPED PINNED host memory and
-// then bumps a sequence word the host spins on: the result reaches the LM loop without a D2H memcpy or a
-// cudaStreamSynchronize round trip (two driver calls and a thread wake-up per launch otherwise).
+// When `host_out` is non-null (every run but a sharded one with the all-reduce callback) the last block also publishes the
+// sums into the handle's HostMailbox (mapped pinned host memory, host_common.h) and then bumps the sequence word the host
+// spins on: the result reaches the LM loop without a D2H memcpy or a cudaStreamSynchronize round trip.
 template <int NV>
 __device__ __forceinline__ void block_reduce_finalize(double* v, double* __restrict__ partial, double* __restrict__ out,
                                                       unsigned int* __restrict__ counter, double* host_out = nullptr,
@@ -981,9 +978,8 @@ struct gsicp_gicp {
   Scratch corr, sqd, mahal, partial, red_out, counter, staging_dev, nn_id, nn_d2;
   int corr_n = 0;
   double* h_red = nullptr;     // pinned [28]
-  unsigned long long* h_map = nullptr;  // mapped pinned: [0..27] sums (as double), [28] sequence word
-  unsigned long long* d_map = nullptr;  // device alias of h_map
-  unsigned long long seq = 0;
+  HostMailbox lin_box;         // linearize / error sums: [0, kRed) as doubles, [kRed] sequence word
+  HostMailbox lm_box;          // LmResult of align_lm_kernel
   void* h_stage = nullptr;     // pinned staging for H2D conversions
   size_t h_stage_cap = 0;
   int shard_count = 1, shard_index = 0;
@@ -991,15 +987,9 @@ struct gsicp_gicp {
   bool src_partial = false;      // sharded covariances: this rank holds only its own source rotations / scales / covariances
   gsicp_allreduce_fn reduce = nullptr;
   void* reduce_user = nullptr;
-  bool host_lm = false;          // GSICP_HOST_LM=1: host-driven LM loop (one launch + one spin-wait per phase)
+  bool host_lm = false;          // gsicp_gicp_set_host_lm: host-driven LM loop (one launch + one spin-wait per phase)
   Scratch lm_partL, lm_partE, lm_barrier;
-  LmResult* h_lm = nullptr;      // mapped pinned result block of align_lm_kernel
-  LmResult* d_lm = nullptr;
   int lm_max_blocks = 0;         // co-resident blocks of align_lm_kernel on this device
-  bool timing = false;
-  double t_cov = 0, t_lin = 0, t_err = 0;
-  int n_lin = 0, n_err = 0;
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };
 
 namespace {
@@ -1044,7 +1034,10 @@ int upload_staged(gsicp_gicp* h, const HostSeg* segs, int nseg) {
     }
   }
   float* stage = (float*)h->h_stage;
-  auto fill = [&](const Chunk& ch) {
+  // Copying chunk k+1 overlaps the DMA of chunk k.  A team of 6 copy threads was measured slower end to end (1.98-2.67 ms
+  // vs 1.51 ms per keyframe: thread start-up and contention with the two Python threads cost more than the extra copy
+  // bandwidth buys).
+  for (const Chunk& ch : chunks) {
     const HostSeg& sg = segs[ch.seg];
     float* out = stage + ch.stage_off;
     if (sg.src_is_f64) {
@@ -1053,69 +1046,10 @@ int upload_staged(gsicp_gicp* h, const HostSeg* segs, int nseg) {
     } else {
       std::memcpy(out, (const float*)sg.src + ch.first, ch.count * sizeof(float));
     }
-  };
-  auto send = [&](const Chunk& ch) -> cudaError_t {
-    return cudaMemcpyAsync((float*)segs[ch.seg].dst + ch.first, stage + ch.stage_off, ch.count * sizeof(float),
-                           cudaMemcpyHostToDevice, h->stream);
-  };
-  // Copying chunk k+1 overlaps the DMA of chunk k.  A small team of copy threads (GSICP_STAGE_THREADS, default 1) can share
-  // the host-side copy; a team of 6 was measured slower end to end (1.98-2.67 ms vs 1.51 ms per keyframe: thread start-up
-  // and contention with the two Python threads cost more than the extra copy bandwidth buys).
-  const int nchunks = (int)chunks.size();
-  static const int team_env = [] { const char* e = getenv("GSICP_STAGE_THREADS"); return e ? atoi(e) : 1; }();
-  const int team = std::min(team_env, nchunks / 2);
-  if (team < 2) {
-    for (const Chunk& ch : chunks) {
-      fill(ch);
-      GSICP_CUDA(send(ch));
-    }
-    return GSICP_OK;
+    GSICP_CUDA(cudaMemcpyAsync((float*)sg.dst + ch.first, out, ch.count * sizeof(float), cudaMemcpyHostToDevice, h->stream));
   }
-  std::vector<std::atomic<int>> done(nchunks);
-  for (auto& d : done) d.store(0, std::memory_order_relaxed);
-  std::atomic<int> next{0};
-  auto work = [&]() {
-    for (int c = next.fetch_add(1); c < nchunks; c = next.fetch_add(1)) {
-      fill(chunks[c]);
-      done[c].store(1, std::memory_order_release);
-    }
-  };
-  std::vector<std::thread> helpers;
-  for (int t = 1; t < team; t++) helpers.emplace_back(work);
-  cudaError_t err = cudaSuccess;
-  int sent = 0;
-  // this thread copies too; after each of its chunks it sends every chunk that is ready, in order
-  for (int c = next.fetch_add(1); c < nchunks; c = next.fetch_add(1)) {
-    fill(chunks[c]);
-    done[c].store(1, std::memory_order_release);
-    while (sent < nchunks && done[sent].load(std::memory_order_acquire)) {
-      if (err == cudaSuccess) err = send(chunks[sent]);
-      sent++;
-    }
-  }
-  for (auto& h2 : helpers) h2.join();
-  for (; sent < nchunks; sent++)
-    if (err == cudaSuccess) err = send(chunks[sent]);
-  GSICP_CUDA(err);
   return GSICP_OK;
 }
-
-struct StageTimer {  // accumulates device time of a stage when timing is enabled
-  gsicp_gicp* h;
-  double* acc;
-  StageTimer(gsicp_gicp* hh, double* a) : h(hh), acc(a) {
-    if (h->timing) cudaEventRecord(h->ev0, h->stream);
-  }
-  void stop() {
-    if (h->timing) {
-      cudaEventRecord(h->ev1, h->stream);
-      cudaEventSynchronize(h->ev1);
-      float ms = 0;
-      cudaEventElapsedTime(&ms, h->ev0, h->ev1);
-      *acc += ms;
-    }
-  }
-};
 
 void shard_range(const gsicp_gicp* h, int n, int& begin, int& end) {
   if (h->shard_count <= 1) {
@@ -1309,35 +1243,7 @@ int ensure_lin_buffers(gsicp_gicp* h) {
     GSICP_CUDA(cudaMemsetAsync(h->counter.ptr, 0, sizeof(unsigned int), h->stream));
   }
   if (!h->h_red) GSICP_CUDA(cudaMallocHost(&h->h_red, kRed * sizeof(double)));
-  if (!h->h_map) {
-    GSICP_CUDA(cudaHostAlloc((void**)&h->h_map, 32 * sizeof(unsigned long long), cudaHostAllocMapped));
-    std::memset(h->h_map, 0, 32 * sizeof(unsigned long long));
-    GSICP_CUDA(cudaHostGetDevicePointer((void**)&h->d_map, h->h_map, 0));
-  }
-  return GSICP_OK;
-}
-
-// Spin until the kernel's last block has published sequence number `seq` into mapped host memory.
-int wait_published(gsicp_gicp* h, unsigned long long seq) {
-  volatile unsigned long long* p = h->h_map + 28;
-  long spins = 0;
-  while (*p != seq) {
-#if defined(__x86_64__)
-    __builtin_ia32_pause();
-#endif
-    if ((++spins & 0xfffff) == 0) {  // every ~1M spins make sure the kernel has not failed
-      const cudaError_t q = cudaStreamQuery(h->stream);
-      if (q != cudaSuccess && q != cudaErrorNotReady) {
-        set_error("kernel failed: %s", cudaGetErrorString(q));
-        return GSICP_ECUDA;
-      }
-      if (q == cudaSuccess && *p != seq) {
-        set_error("reduction result was not published");
-        return GSICP_ECUDA;
-      }
-    }
-  }
-  return GSICP_OK;
+  return h->lin_box.ensure((kRed + 1) * sizeof(unsigned long long));
 }
 
 // ---- sum-merge of a sharded array over the exchange group (getters of sharded runs; not on the LM path) ----
@@ -1415,6 +1321,27 @@ int comm_take_seq(gsicp_gicp* h, unsigned long long reserve, unsigned long long*
   return GSICP_OK;
 }
 
+// The n sums of a linearize / error launch into h->h_red.  Single-GPU and in-kernel-exchange runs read them from the mailbox
+// the kernel published into; a sharded run with the all-reduce callback sums red_out over the ranks and copies it back.
+int collect_sums(gsicp_gicp* h, int n, bool direct, unsigned long long seq) {
+  if (h->shard_count > 1 && h->reduce) {
+    const int rc = h->reduce(h->reduce_user, h->red_out.as<double>(), n, (void*)h->stream);
+    if (rc != 0) {
+      set_error("all-reduce callback failed (%d)", rc);
+      return GSICP_ECUDA;
+    }
+  }
+  if (direct) {
+    GSICP_CUDA(cudaGetLastError());
+    if (int e = h->lin_box.wait(kRed, seq, h->stream, "GICP reduction")) return e;
+    std::memcpy(h->h_red, h->lin_box.host, n * sizeof(double));
+  } else {
+    GSICP_CUDA(cudaMemcpyAsync(h->h_red, h->red_out.ptr, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
+    GSICP_CUDA(cudaStreamSynchronize(h->stream));
+  }
+  return GSICP_OK;
+}
+
 // fgi:296-352.  H may be null (error only).
 int run_linearize(gsicp_gicp* h, const Iso& x, double H[6][6], double b[6], double* err) {
   if (int e = ensure_lin_buffers(h)) return e;
@@ -1424,7 +1351,6 @@ int run_linearize(gsicp_gicp* h, const Iso& x, double H[6][6], double b[6], doub
     GSICP_CUDA(cudaMemsetAsync(h->sqd.ptr, 0, (size_t)(h->src.n + 1) * 4, h->stream));
     h->corr_n = h->src.n;
   }
-  StageTimer tm(h, &h->t_lin);
   int begin, end;
   shard_range(h, h->src.n, begin, end);
   LinArgs a;
@@ -1435,10 +1361,10 @@ int run_linearize(gsicp_gicp* h, const Iso& x, double H[6][6], double b[6], doub
   a.corr = h->corr.as<int32_t>(); a.sqd = h->sqd.as<float>(); a.mahal = h->mahal.as<double>();
   a.partial = h->partial.as<double>(); a.out = h->red_out.as<double>(); a.counter = h->counter.as<unsigned int>();
   const bool xchg = h->shard_count > 1 && h->comm;  // in-kernel exchange: the published sums are already global
-  const bool direct = (h->shard_count <= 1 || xchg) && !h->timing;  // publish straight into mapped host memory
-  a.host_out = direct ? (double*)h->d_map : nullptr;
-  a.host_seq = direct ? (volatile unsigned long long*)(h->d_map + 28) : nullptr;
-  a.seq = ++h->seq;
+  const bool direct = h->shard_count <= 1 || xchg;   // publish straight into mapped host memory
+  a.host_out = direct ? (double*)h->lin_box.dev : nullptr;
+  a.host_seq = direct ? (volatile unsigned long long*)(h->lin_box.dev + kRed) : nullptr;
+  a.seq = ++h->lin_box.seq;
   a.comm = CommView();
   a.xseq = 0;
   if (xchg) {
@@ -1456,23 +1382,7 @@ int run_linearize(gsicp_gicp* h, const Iso& x, double H[6][6], double b[6], doub
                  a.src_xyz, a.corr, a.sqd);
   }
   GSICP_LAUNCH(linearize_kernel, blocks, kLinBlock, 0, h->stream, make_pose(x), a); }
-  if (h->shard_count > 1 && h->reduce) {
-    const int rc = h->reduce(h->reduce_user, h->red_out.as<double>(), kRed, (void*)h->stream);
-    if (rc != 0) {
-      set_error("all-reduce callback failed (%d)", rc);
-      return GSICP_ECUDA;
-    }
-  }
-  if (direct) {
-    GSICP_CUDA(cudaGetLastError());
-    if (int e = wait_published(h, a.seq)) return e;
-    std::memcpy(h->h_red, h->h_map, kRed * sizeof(double));
-  } else {
-    GSICP_CUDA(cudaMemcpyAsync(h->h_red, h->red_out.ptr, kRed * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    tm.stop();
-    GSICP_CUDA(cudaStreamSynchronize(h->stream));
-  }
-  h->n_lin++;
+  if (int e = collect_sums(h, kRed, direct, a.seq)) return e;
   if (H && b) {
     int o = 0;
     for (int r = 0; r < 6; r++)
@@ -1489,7 +1399,6 @@ int run_linearize(gsicp_gicp* h, const Iso& x, double H[6][6], double b[6], doub
 
 int run_error(gsicp_gicp* h, const Iso& x, double* err) {  // fgi:355-378
   if (int e = ensure_lin_buffers(h)) return e;
-  StageTimer tm(h, &h->t_err);
   int begin, end;
   shard_range(h, h->src.n, begin, end);
   ErrArgs a;
@@ -1498,10 +1407,10 @@ int run_error(gsicp_gicp* h, const Iso& x, double* err) {  // fgi:355-378
   a.corr = h->corr.as<int32_t>(); a.mahal = h->mahal.as<double>();
   a.partial = h->partial.as<double>(); a.out = h->red_out.as<double>(); a.counter = h->counter.as<unsigned int>();
   const bool xchg = h->shard_count > 1 && h->comm;
-  const bool direct = (h->shard_count <= 1 || xchg) && !h->timing;
-  a.host_out = direct ? (double*)h->d_map : nullptr;
-  a.host_seq = direct ? (volatile unsigned long long*)(h->d_map + 28) : nullptr;
-  a.seq = ++h->seq;
+  const bool direct = h->shard_count <= 1 || xchg;
+  a.host_out = direct ? (double*)h->lin_box.dev : nullptr;
+  a.host_seq = direct ? (volatile unsigned long long*)(h->lin_box.dev + kRed) : nullptr;
+  a.seq = ++h->lin_box.seq;
   a.comm = CommView();
   a.xseq = 0;
   if (xchg) {
@@ -1512,20 +1421,7 @@ int run_error(gsicp_gicp* h, const Iso& x, double* err) {  // fgi:355-378
   if (blocks < 1) blocks = 1;
   { ProfScope ps(kProfError, h->stream);
   GSICP_LAUNCH(error_kernel, blocks, kLinBlock, 0, h->stream, make_pose(x), a); }
-  if (h->shard_count > 1 && h->reduce) {
-    const int rc = h->reduce(h->reduce_user, h->red_out.as<double>(), 1, (void*)h->stream);
-    if (rc != 0) return GSICP_ECUDA;
-  }
-  if (direct) {
-    GSICP_CUDA(cudaGetLastError());
-    if (int e = wait_published(h, a.seq)) return e;
-    h->h_red[0] = *(const double*)h->h_map;
-  } else {
-    GSICP_CUDA(cudaMemcpyAsync(h->h_red, h->red_out.ptr, sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    tm.stop();
-    GSICP_CUDA(cudaStreamSynchronize(h->stream));
-  }
-  h->n_err++;
+  if (int e = collect_sums(h, 1, direct, a.seq)) return e;
   *err = h->h_red[0];
   return GSICP_OK;
 }
@@ -1575,11 +1471,7 @@ int run_align_device(gsicp_gicp* h, Iso& x0) {
     GSICP_CUDA(cudaMemsetAsync(h->sqd.ptr, 0, (size_t)(h->src.n + 1) * 4, h->stream));
     h->corr_n = h->src.n;
   }
-  if (!h->h_lm) {
-    GSICP_CUDA(cudaHostAlloc((void**)&h->h_lm, sizeof(LmResult), cudaHostAllocMapped));
-    std::memset(h->h_lm, 0, sizeof(LmResult));
-    GSICP_CUDA(cudaHostGetDevicePointer((void**)&h->d_lm, h->h_lm, 0));
-  }
+  if (int e = h->lm_box.ensure(sizeof(LmResult))) return e;
   if (h->lm_max_blocks == 0) {
     int dev = 0, sms = 0;
     GSICP_CUDA(cudaGetDevice(&dev));
@@ -1617,8 +1509,8 @@ int run_align_device(gsicp_gicp* h, Iso& x0) {
   a.max_iterations = h->max_iterations; a.lm_max_iterations = h->lm_max_iterations;
   a.rot_eps = h->rot_eps; a.trans_eps = h->trans_eps; a.init_lambda_factor = h->lm_init_lambda_factor;
   a.guess = x0;
-  a.result = h->d_lm;
-  a.seq = ++h->seq;
+  a.result = reinterpret_cast<LmResult*>(h->lm_box.dev);
+  a.seq = ++h->lm_box.seq;
   static const int s_marks = [] { const char* e = getenv("GSICP_LM_MARKS"); return e ? atoi(e) : 0; }();
   a.marks = s_marks;
   {
@@ -1626,26 +1518,9 @@ int run_align_device(gsicp_gicp* h, Iso& x0) {
     GSICP_LAUNCH(align_lm_kernel, blocks, kLmBlock, 0, h->stream, a);
   }
   GSICP_CUDA(cudaGetLastError());
-  // spin on the sequence word the kernel publishes into mapped pinned memory
-  volatile unsigned long long* p = &h->h_lm->seq;
-  long spins = 0;
-  while (*p != a.seq) {
-#if defined(__x86_64__)
-    __builtin_ia32_pause();
-#endif
-    if ((++spins & 0xfffff) == 0) {
-      const cudaError_t q = cudaStreamQuery(h->stream);
-      if (q != cudaSuccess && q != cudaErrorNotReady) {
-        set_error("align kernel failed: %s", cudaGetErrorString(q));
-        return GSICP_ECUDA;
-      }
-      if (q == cudaSuccess && *p != a.seq) {
-        set_error("align result was not published");
-        return GSICP_ECUDA;
-      }
-    }
-  }
-  const LmResult r = *h->h_lm;
+  static_assert(offsetof(LmResult, seq) % sizeof(unsigned long long) == 0, "LmResult::seq must be a mailbox word");
+  if (int e = h->lm_box.wait(offsetof(LmResult, seq) / sizeof(unsigned long long), a.seq, h->stream, "align result")) return e;
+  const LmResult r = *reinterpret_cast<const LmResult*>(h->lm_box.host);
   if (s_marks && r.n_marks > 1) {
     fprintf(stderr, "[lm marks] total %.1f us:", (double)(r.marks[r.n_marks - 1] - r.marks[0]) * 1e-3);
     for (int i = 1; i < r.n_marks; i++) fprintf(stderr, " %.1f", (double)(r.marks[i] - r.marks[i - 1]) * 1e-3);
@@ -1658,8 +1533,6 @@ int run_align_device(gsicp_gicp* h, Iso& x0) {
   h->lm_lambda = r.lambda;
   h->converged = r.converged != 0;
   h->nr_iterations = r.iterations - 1;
-  h->n_lin = r.n_lin;
-  h->n_err = r.n_err;
   // final_hessian_ is only assigned by an accepted step (lsq:169); it keeps its previous value otherwise
   if (r.n_err > 0) {
     bool any = false;
@@ -1702,11 +1575,7 @@ gsicp_gicp* gsicp_gicp_create(void) {
   gsicp_gicp* h = new gsicp_gicp();
   for (int i = 0; i < 16; i++) h->final_transformation[i] = (i % 5 == 0) ? 1.f : 0.f;
   for (int i = 0; i < 36; i++) h->final_hessian[i] = (i % 7 == 0) ? 1.0 : 0.0;
-  const char* t = std::getenv("GSICP_TIMING");
-  h->timing = t && t[0] == '1';
-  const char* hl = std::getenv("GSICP_HOST_LM");
-  h->host_lm = hl && hl[0] == '1';
-  if (cudaEventCreate(&h->ev0) != cudaSuccess || cudaEventCreate(&h->ev1) != cudaSuccess) {
+  if (cudaFree(nullptr) != cudaSuccess) {  // initialises the context
     set_error("gsicp_gicp_create: no usable CUDA device (%s)", cudaGetErrorString(cudaGetLastError()));
     delete h;
     return nullptr;
@@ -1727,12 +1596,10 @@ void gsicp_gicp_destroy(gsicp_gicp* h) {
   }
   fr(h->corr); fr(h->sqd); fr(h->mahal); fr(h->partial); fr(h->red_out); fr(h->counter); fr(h->staging_dev); fr(h->nn_id); fr(h->nn_d2);
   fr(h->lm_partL); fr(h->lm_partE); fr(h->lm_barrier);
-  if (h->h_lm) cudaFreeHost(h->h_lm);
+  h->lm_box.release();
+  h->lin_box.release();
   if (h->h_red) cudaFreeHost(h->h_red);
-  if (h->h_map) cudaFreeHost(h->h_map);
   if (h->h_stage) cudaFreeHost(h->h_stage);
-  if (h->ev0) cudaEventDestroy(h->ev0);
-  if (h->ev1) cudaEventDestroy(h->ev1);
   delete h;
 }
 
@@ -1810,13 +1677,9 @@ int gsicp_gicp_align(gsicp_gicp* h, const float guess[16], float out[16]) {
     return GSICP_ESTATE;
   }
   h->converged = false;
-  h->t_cov = h->t_lin = h->t_err = 0;
-  h->n_lin = h->n_err = 0;
   // fgi:225-240: lazily compute missing covariances
   if (h->src.cov_n != h->src.n) {
-    StageTimer tm(h, &h->t_cov);
     if (int e = compute_covariances(h, h->src, true, false)) return e;
-    tm.stop();
     h->corr_n = -1;
   }
   if (h->tgt.cov_n != h->tgt.n) {
@@ -1838,9 +1701,9 @@ int gsicp_gicp_align(gsicp_gicp* h, const float guess[16], float out[16]) {
   // The persistent kernel (one block per SM) wins where launch / wait latency dominates; above kLmPersistentMax points per
   // rank the phases are throughput-bound and the full-occupancy kernels of the host-driven loop are faster
   // (in a sharded run their last block exchanges through the peers' segments as well: no host-side collective either way).
-  if (!h->host_lm && !h->timing && (h->shard_count <= 1 || h->comm) && (le - lb) <= kLmPersistentMax) {
+  if (!h->host_lm && (h->shard_count <= 1 || h->comm) && (le - lb) <= kLmPersistentMax) {
     // device-resident LM loop: one persistent kernel, zero host round trips inside the loop
-    if (h->d_lm) std::memset(h->h_lm->H, 0, sizeof(h->h_lm->H));
+    if (h->lm_box.host) std::memset(reinterpret_cast<LmResult*>(h->lm_box.host)->H, 0, sizeof(LmResult::H));
     iters = run_align_device(h, x0);
     if (iters < 0) return iters;
   } else {
@@ -2011,12 +1874,6 @@ int gsicp_gicp_set_comm(gsicp_gicp* h, gsicp_comm* comm) {
   h->reduce_user = nullptr;
   h->corr_n = -1;
   h->src.clear_cov();
-  return GSICP_OK;
-}
-
-int gsicp_gicp_last_timing(gsicp_gicp* h, double out[5]) {
-  H_CHECK(h);
-  out[0] = h->t_cov; out[1] = h->t_lin; out[2] = h->t_err; out[3] = h->n_lin; out[4] = h->n_err;
   return GSICP_OK;
 }
 

@@ -69,4 +69,19 @@ struct Scratch {
   T* as() const { return reinterpret_cast<T*>(ptr); }
 };
 
+// Mapped pinned words a kernel publishes a small result into (a count, a reduction, the LM result), then a sequence word
+// the host spins on.  The host gets the result without a D2H memcpy + cudaStreamSynchronize round trip (two driver calls
+// and a thread wake-up per result otherwise).  Not thread-safe: each owner serialises its launches and waits itself.
+struct HostMailbox {
+  unsigned long long* host = nullptr;  // mapped pinned, zeroed on first use
+  unsigned long long* dev = nullptr;   // device alias of host
+  unsigned long long seq = 0;          // last sequence number handed out
+  int ensure(size_t bytes);
+  // Spins until host[word] == s.  The fast path makes no driver call; every ~1M spins the stream is queried so that a
+  // failed kernel ("<what> failed: ...") or a finished stream that never published s ("<what> was not published")
+  // returns GSICP_ECUDA instead of hanging.
+  int wait(size_t word, unsigned long long s, cudaStream_t stream, const char* what) const;
+  void release();
+};
+
 }  // namespace gsicp

@@ -12,9 +12,9 @@
 //                          compacted (xyz, normalised rotation, exp(scaling)) written straight into device buffers that
 //                          FastGICP.set_input_target / set_target_covariances_fromqs take without leaving the GPU (the
 //                          reference goes GPU -> CPU -> shared memory -> numpy -> pybind -> kd-tree at every tracking keyframe)
-#include <cub/cub.cuh>
 #include <mutex>
 #include "host_common.h"
+#include "scan.cuh"
 
 namespace gsicp {
 
@@ -126,55 +126,9 @@ trackable_target_kernel(int P, TrackFlag f, const int* __restrict__ excl, const 
 struct TableScratch {
   std::mutex mu;
   Scratch excl, cub_tmp;
-  unsigned long long* h_map = nullptr;
-  unsigned long long* d_map = nullptr;
-  unsigned long long seq = 0;
+  HostMailbox box;  // [0] row count, [1] sequence word
 };
 static TableScratch g_tab;
-
-static int table_ready(int rows) {
-  if (!g_tab.h_map) {
-    GSICP_CUDA(cudaHostAlloc((void**)&g_tab.h_map, 2 * sizeof(unsigned long long), cudaHostAllocMapped));
-    g_tab.h_map[0] = g_tab.h_map[1] = 0;
-    GSICP_CUDA(cudaHostGetDevicePointer((void**)&g_tab.d_map, g_tab.h_map, 0));
-  }
-  return g_tab.excl.ensure((size_t)rows * sizeof(int));
-}
-
-template <typename Flag>
-static int table_scan(int rows, Flag flag, cudaStream_t stream) {
-  cub::CountingInputIterator<int> counting(0);
-  cub::TransformInputIterator<int, Flag, cub::CountingInputIterator<int>> flags(counting, flag);
-  size_t tmp = 0;
-  cub::DeviceScan::ExclusiveSum(nullptr, tmp, flags, g_tab.excl.as<int>(), rows, stream);
-  if (int e = g_tab.cub_tmp.ensure(tmp)) return e;
-  tmp = g_tab.cub_tmp.cap;
-  GSICP_CUDA(cub::DeviceScan::ExclusiveSum(g_tab.cub_tmp.ptr, tmp, flags, g_tab.excl.as<int>(), rows, stream));
-  return GSICP_OK;
-}
-
-static int table_wait_count(unsigned long long seq, cudaStream_t stream, long long* count) {
-  volatile unsigned long long* pm = g_tab.h_map;
-  long spins = 0;
-  while (pm[1] != seq) {
-#if defined(__x86_64__)
-    __builtin_ia32_pause();
-#endif
-    if ((++spins & 0xfffff) == 0) {
-      const cudaError_t q = cudaStreamQuery(stream);
-      if (q != cudaSuccess && q != cudaErrorNotReady) {
-        set_error("table kernel failed: %s", cudaGetErrorString(q));
-        return GSICP_ECUDA;
-      }
-      if (q == cudaSuccess && pm[1] != seq) {
-        set_error("row count was not published");
-        return GSICP_ECUDA;
-      }
-    }
-  }
-  *count = (long long)pm[0];
-  return GSICP_OK;
-}
 
 }  // namespace gsicp
 
@@ -221,8 +175,9 @@ extern "C" long long gsicp_table_compact(int rows, const uint8_t* d_keep, int n_
   if (rows == 0) return 0;
   cudaStream_t stream = (cudaStream_t)stream_v;
   std::lock_guard<std::mutex> lock(g_tab.mu);
-  if (int e = table_ready(rows)) return e;
-  if (int e = table_scan(rows, KeepFlag{d_keep}, stream)) return e;
+  HostMailbox& box = g_tab.box;
+  if (int e = box.ensure(2 * sizeof(unsigned long long))) return e;
+  if (int e = flag_exclusive_scan<int>(rows, KeepFlag{d_keep}, g_tab.excl, g_tab.cub_tmp, stream)) return e;
   CompactArrays a;
   a.n = n_arrays;
   for (int k = 0; k < n_arrays; k++) {
@@ -234,12 +189,11 @@ extern "C" long long gsicp_table_compact(int rows, const uint8_t* d_keep, int n_
     a.dst[k] = (char*)d_dst[k];
     a.row_bytes[k] = row_bytes[k];
   }
-  const unsigned long long seq = ++g_tab.seq;
-  GSICP_LAUNCH(compact_rows_kernel, (rows + 255) / 256, 256, 0, stream, rows, d_keep, g_tab.excl.as<int>(), a, g_tab.d_map, seq);
+  const unsigned long long seq = ++box.seq;
+  GSICP_LAUNCH(compact_rows_kernel, (rows + 255) / 256, 256, 0, stream, rows, d_keep, g_tab.excl.as<int>(), a, box.dev, seq);
   GSICP_CUDA(cudaGetLastError());
-  long long count = 0;
-  if (int e = table_wait_count(seq, stream, &count)) return e;
-  return count;
+  if (int e = box.wait(1, seq, stream, "compacted row count")) return e;
+  return (long long)box.host[0];
 }
 
 extern "C" long long gsicp_trackable_target(int P, const float* d_xyz, const float* d_rotation_raw, const float* d_scaling_raw,
@@ -253,14 +207,14 @@ extern "C" long long gsicp_trackable_target(int P, const float* d_xyz, const flo
   }
   cudaStream_t stream = (cudaStream_t)stream_v;
   std::lock_guard<std::mutex> lock(g_tab.mu);
-  if (int e = table_ready(P)) return e;
+  HostMailbox& box = g_tab.box;
+  if (int e = box.ensure(2 * sizeof(unsigned long long))) return e;
   const TrackFlag f{d_opacity_raw, d_trackable, opacity_th};
-  if (int e = table_scan(P, f, stream)) return e;
-  const unsigned long long seq = ++g_tab.seq;
+  if (int e = flag_exclusive_scan<int>(P, f, g_tab.excl, g_tab.cub_tmp, stream)) return e;
+  const unsigned long long seq = ++box.seq;
   GSICP_LAUNCH(trackable_target_kernel, (P + 255) / 256, 256, 0, stream, P, f, g_tab.excl.as<int>(), d_xyz, d_rotation_raw,
-               d_scaling_raw, d_out_xyz, d_out_rot, d_out_scale, g_tab.d_map, seq);
+               d_scaling_raw, d_out_xyz, d_out_rot, d_out_scale, box.dev, seq);
   GSICP_CUDA(cudaGetLastError());
-  long long count = 0;
-  if (int e = table_wait_count(seq, stream, &count)) return e;
-  return count;
+  if (int e = box.wait(1, seq, stream, "trackable target count")) return e;
+  return (long long)box.host[0];
 }

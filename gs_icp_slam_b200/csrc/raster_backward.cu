@@ -18,12 +18,12 @@
 //
 // per-Gaussian backward: computeCov2D backward and the preprocess backward are one kernel (the
 // intermediate dL_dcov3D / dL_dmeans never round-trip through HBM between two launches).
-#include <cub/cub.cuh>
 #include <cstdlib>
 #include <mutex>
 #include "host_common.h"
 #include "raster_common.cuh"
 #include "comm.cuh"
+#include "scan.cuh"
 
 namespace gsicp {
 
@@ -746,46 +746,21 @@ struct BwdShared {
   gsicp_allreduce_f32_fn fn = nullptr;
   void* user = nullptr;
   Scratch excl, dense, cub_tmp;
-  unsigned long long* h_map = nullptr;
-  unsigned long long* d_map = nullptr;
-  unsigned long long seq = 0;
+  HostMailbox box;  // [0] visible count V, [1] sequence word
 };
 static BwdShared g_bwd;
 
 static int allreduce_visible_moments(int P, const int32_t* d_radii, float* moments, cudaStream_t stream) {
   std::lock_guard<std::mutex> lock(g_bwd.mu);
-  if (!g_bwd.h_map) {
-    GSICP_CUDA(cudaHostAlloc((void**)&g_bwd.h_map, 2 * sizeof(unsigned long long), cudaHostAllocMapped));
-    g_bwd.h_map[0] = g_bwd.h_map[1] = 0;
-    GSICP_CUDA(cudaHostGetDevicePointer((void**)&g_bwd.d_map, g_bwd.h_map, 0));
-  }
-  if (int e = g_bwd.excl.ensure((size_t)P * 4)) return e;
-  cub::CountingInputIterator<int> counting(0);
-  cub::TransformInputIterator<uint32_t, VisibleFlag, cub::CountingInputIterator<int>> flags(counting, VisibleFlag{d_radii});
-  size_t tmp = 0;
-  cub::DeviceScan::ExclusiveSum(nullptr, tmp, flags, g_bwd.excl.as<uint32_t>(), P, stream);
-  if (int e = g_bwd.cub_tmp.ensure(tmp)) return e;
-  tmp = g_bwd.cub_tmp.cap;
-  GSICP_CUDA(cub::DeviceScan::ExclusiveSum(g_bwd.cub_tmp.ptr, tmp, flags, g_bwd.excl.as<uint32_t>(), P, stream));
-  const unsigned long long seq = ++g_bwd.seq;
+  HostMailbox& box = g_bwd.box;
+  if (int e = box.ensure(2 * sizeof(unsigned long long))) return e;
+  if (int e = flag_exclusive_scan<uint32_t>(P, VisibleFlag{d_radii}, g_bwd.excl, g_bwd.cub_tmp, stream)) return e;
+  const unsigned long long seq = ++box.seq;
   GSICP_LAUNCH(publish_visible_kernel, 1, 1, 0, stream, P, g_bwd.excl.as<uint32_t>(), d_radii,
-               (volatile unsigned long long*)g_bwd.d_map, seq);
+               (volatile unsigned long long*)box.dev, seq);
   GSICP_CUDA(cudaGetLastError());
-  volatile unsigned long long* pm = g_bwd.h_map;
-  long spins = 0;
-  while (pm[1] != seq) {
-#if defined(__x86_64__)
-    __builtin_ia32_pause();
-#endif
-    if ((++spins & 0xfffff) == 0) {
-      const cudaError_t q = cudaStreamQuery(stream);
-      if (q != cudaSuccess && q != cudaErrorNotReady) {
-        set_error("rasterizer backward failed: %s", cudaGetErrorString(q));
-        return GSICP_ECUDA;
-      }
-    }
-  }
-  const size_t V = (size_t)pm[0];
+  if (int e = box.wait(1, seq, stream, "visible Gaussian count")) return e;
+  const size_t V = (size_t)box.host[0];
   if (V == 0) return GSICP_OK;
   if (int e = g_bwd.dense.ensure(V * kG * sizeof(float))) return e;
   GSICP_LAUNCH(moments_compact_kernel<true>, (P + 255) / 256, 256, 0, stream, P, d_radii, g_bwd.excl.as<uint32_t>(), moments,

@@ -461,9 +461,7 @@ constexpr int kMaxDevices = 32;
 struct FwdScratch {
   std::mutex mu;
   Scratch per_gaussian, per_instance, cub_tmp;
-  unsigned long long* h_map = nullptr;  // mapped pinned: [0] = num_rendered, [1] = sequence word, [2] = largest tile
-  unsigned long long* d_map = nullptr;
-  unsigned long long seq = 0;
+  HostMailbox box;  // [0] num_rendered, [1] sequence word, [2] largest tile, [3] tiles of >= kSmallTileCap instances
   bool sort_attr_set = false;  // cudaFuncSetAttribute of the big tile sort, per device
 };
 static FwdScratch g_fwd_dev[kMaxDevices];
@@ -521,11 +519,8 @@ extern "C" int gsicp_raster_forward(const gsicp_raster_args* args, float* d_out_
   }
   FwdScratch& g_fwd = g_fwd_dev[dev];
   std::lock_guard<std::mutex> lock(g_fwd.mu);
-  if (!g_fwd.h_map) {
-    GSICP_CUDA(cudaHostAlloc((void**)&g_fwd.h_map, 4 * sizeof(unsigned long long), cudaHostAllocMapped));
-    g_fwd.h_map[0] = g_fwd.h_map[1] = g_fwd.h_map[2] = 0;
-    GSICP_CUDA(cudaHostGetDevicePointer((void**)&g_fwd.d_map, g_fwd.h_map, 0));
-  }
+  HostMailbox& box = g_fwd.box;
+  if (int e = box.ensure(4 * sizeof(unsigned long long))) return e;
 
   int R = 0;
   unsigned long long max_tile = 0;
@@ -566,40 +561,21 @@ extern "C" int gsicp_raster_forward(const gsicp_raster_args* args, float* d_out_
     // The Python API returns num_rendered as a host int (DGR/diff_gaussian_rasterization/__init__.py:96) and the instance
     // buffers are sized by it (rasterizer_impl.cu:286-287 does a blocking 4-byte memcpy).  Here the scan kernel publishes
     // it into mapped pinned memory and the host spins on a sequence word.
-    const unsigned long long seq = ++g_fwd.seq;
+    const unsigned long long seq = ++box.seq;
     {
       ProfScope ps(kProfDepthSort, stream);  // slot reused: "tile_scan"
       GSICP_LAUNCH(tile_scan_kernel, 1, 1024, 0, stream, tiles, tile_count, img.ranges, cursor, seg_begin, seg_end,
-                   img.tile_order, (volatile unsigned long long*)g_fwd.d_map, seq);
+                   img.tile_order, (volatile unsigned long long*)box.dev, seq);
     }
     GSICP_CUDA(cudaGetLastError());
-    {
-      volatile unsigned long long* pm = g_fwd.h_map;
-      long spins = 0;
-      while (pm[1] != seq) {
-#if defined(__x86_64__)
-        __builtin_ia32_pause();
-#endif
-        if ((++spins & 0xfffff) == 0) {
-          const cudaError_t q = cudaStreamQuery(stream);
-          if (q != cudaSuccess && q != cudaErrorNotReady) {
-            set_error("rasterizer forward failed before binning: %s", cudaGetErrorString(q));
-            return GSICP_ECUDA;
-          }
-          if (q == cudaSuccess && pm[1] != seq) {
-            set_error("instance count was not published");
-            return GSICP_ECUDA;
-          }
-        }
-      }
-      if (pm[0] > 0x7fffffffull) {
-        set_error("gsicp_raster_forward: instance count overflow");
-        return GSICP_EINVAL;
-      }
-      R = (int)pm[0];
-      max_tile = pm[2];
-      n_big = (int)pm[3];
+    if (int e = box.wait(1, seq, stream, "rasterizer instance count")) return e;
+    if (box.host[0] > 0x7fffffffull) {
+      set_error("gsicp_raster_forward: instance count overflow");
+      return GSICP_EINVAL;
     }
+    R = (int)box.host[0];
+    max_tile = box.host[2];
+    n_big = (int)box.host[3];
   } else {
     GSICP_CUDA(cudaMemsetAsync(img.ranges, 0, sizeof(uint2) * tiles, stream));
   }

@@ -253,11 +253,6 @@ class FastGICP:
         check(lib.gsicp_gicp_compute_error(self._h, p.ctypes.data, C.byref(e)), "compute_error")
         return e.value
 
-    def last_timing(self):
-        t = (C.c_double * 5)()
-        check(lib.gsicp_gicp_last_timing(self._h, t))
-        return dict(cov_ms=t[0], linearize_ms=t[1], error_ms=t[2], n_linearize=int(t[3]), n_error=int(t[4]))
-
     def set_stream(self, cuda_stream):
         check(lib.gsicp_gicp_set_stream(self._h, int(cuda_stream)))
         self._stream_ptr = int(cuda_stream)

@@ -255,10 +255,6 @@ int gsicp_gicp_set_stream(gsicp_gicp*, void* stream);
 /* Test / A-B hook: 1 = drive the LM loop from the host (one launch + one wait per linearize / compute_error), 0 (default) =
  * the device-resident loop (one persistent kernel per align, lsq_registration_impl.hpp:53-173 on the GPU).  Same results. */
 int gsicp_gicp_set_host_lm(gsicp_gicp* h, int on);
-/* Timing of the last align(): milliseconds spent in each stage, measured with CUDA events on the
- * handle's stream: [0]=source covariance, [1]=linearize total, [2]=compute_error total,
- * [3]=number of linearize launches, [4]=number of compute_error launches. */
-int gsicp_gicp_last_timing(gsicp_gicp*, double out[5]);
 
 /* ---- fused mapping loss (SURVEY.md §8f row N2; the caller side of the rasterizer) ----------------------------------
  * Replaces utils/loss_utils.py:17-20 (l1_loss), :38-69 (ssim/_ssim) and their combination in mp_Mapper.py:225-242:
