@@ -19,8 +19,6 @@ if not os.path.exists(LIB_PATH):
 lib = C.CDLL(LIB_PATH, mode=C.RTLD_GLOBAL)
 
 ALLOC_FN = C.CFUNCTYPE(C.c_void_p, C.c_size_t, C.c_void_p)
-ALLREDUCE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p)
-ALLREDUCE_F32_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p)
 
 
 class RasterArgs(C.Structure):
@@ -78,7 +76,6 @@ _sig("gsicp_prof_read", i32, [i32, f64p, C.POINTER(C.c_long)])
 
 _sig("gsicp_raster_forward", i32, [C.POINTER(RasterArgs), vp, vp, vp, vp, ALLOC_FN, ALLOC_FN, ALLOC_FN, vp, vp])
 _sig("gsicp_raster_backward_work_bytes", C.c_size_t, [i32])
-_sig("gsicp_raster_set_allreduce", i32, [ALLREDUCE_F32_FN, vp])
 _sig("gsicp_raster_backward", i32, [C.POINTER(RasterArgs), i32, vp, vp, vp, vp, vp, vp] + [vp] * 8 + [vp, vp])
 _sig("gsicp_raster_export_binning", i32, [C.POINTER(RasterArgs), i32, vp, vp, vp, vp, vp])
 _sig("gsicp_mark_visible", i32, [i32, vp, vp, vp, vp, vp])
@@ -119,7 +116,6 @@ _sig("gsicp_gicp_get_final_hessian", i32, [vp, vp])
 _sig("gsicp_gicp_get_source_correspondence", i32, [vp, vp, vp])
 _sig("gsicp_gicp_linearize", i32, [vp, vp, vp, vp, vp])
 _sig("gsicp_gicp_compute_error", i32, [vp, vp, vp])
-_sig("gsicp_gicp_set_shard", i32, [vp, i32, i32, ALLREDUCE_FN, vp])
 _sig("gsicp_gicp_set_stream", i32, [vp, vp])
 _sig("gsicp_gicp_set_host_lm", i32, [vp, i32])
 _sig("gsicp_gicp_set_source_filter_device", i32, [vp, i32, vp, i32])

@@ -227,17 +227,13 @@ __device__ __forceinline__ double warp_sum_d(double v) {
 }
 
 // block-level reduction of NV doubles per thread into partial[blockIdx][NV]; the last block to finish
-// sums the partials in block order (deterministic) into out[NV].
-//
-// When `host_out` is non-null (every run but a sharded one with the all-reduce callback) the last block also publishes the
-// sums into the handle's HostMailbox (mapped pinned host memory, host_common.h) and then bumps the sequence word the host
-// spins on: the result reaches the LM loop without a D2H memcpy or a cudaStreamSynchronize round trip.
+// sums the partials in block order (deterministic), publishes the sums into the handle's HostMailbox (mapped pinned host
+// memory, host_common.h) and then bumps the sequence word the host spins on: the result reaches the LM loop without a D2H
+// memcpy or a cudaStreamSynchronize round trip.
 template <int NV>
-__device__ __forceinline__ void block_reduce_finalize(double* v, double* __restrict__ partial, double* __restrict__ out,
-                                                      unsigned int* __restrict__ counter, double* host_out = nullptr,
-                                                      volatile unsigned long long* host_seq = nullptr,
-                                                      unsigned long long seq = 0, CommView comm = CommView(),
-                                                      unsigned long long xseq = 0) {
+__device__ __forceinline__ void block_reduce_finalize(double* v, double* __restrict__ partial, unsigned int* __restrict__ counter,
+                                                      double* host_out, volatile unsigned long long* host_seq,
+                                                      unsigned long long seq, CommView comm, unsigned long long xseq) {
   __shared__ double s_red[kLinBlock / 32][NV];
   __shared__ double s_tot[NV];
   __shared__ bool s_last;
@@ -275,20 +271,13 @@ __device__ __forceinline__ void block_reduce_finalize(double* v, double* __restr
       comm_lm_publish(comm, xseq, s_tot, NV);
       comm_lm_collect(comm, xseq, s_tot, NV);  // a lost peer leaves the local sums in place after the poll budget
     }
-    if (threadIdx.x < NV) {
-      out[threadIdx.x] = s_tot[threadIdx.x];
-      if (host_out) host_out[threadIdx.x] = s_tot[threadIdx.x];
-    }
-    if (host_out) {
-      __threadfence_system();
-      __syncthreads();  // s_last is block-uniform
-    }
+    if (threadIdx.x < NV) host_out[threadIdx.x] = s_tot[threadIdx.x];
+    __threadfence_system();
+    __syncthreads();  // s_last is block-uniform
     if (threadIdx.x == 0) {
       *counter = 0u;  // ready for the next launch
-      if (host_seq) {
-        *host_seq = seq;
-        __threadfence_system();
-      }
+      *host_seq = seq;
+      __threadfence_system();
     }
   }
 }
@@ -304,9 +293,8 @@ struct LinArgs {
   float* sqd;
   double* mahal;           // [6 * n_src]
   double* partial;
-  double* out;             // [28]
   unsigned int* counter;
-  double* host_out;        // mapped pinned [28] or null
+  double* host_out;        // mapped pinned [28]
   volatile unsigned long long* host_seq;
   unsigned long long seq;
   CommView comm;             // multi-GPU: exchange inside the last block
@@ -366,24 +354,6 @@ fitness_kernel(int n, const float* __restrict__ sqd, double max_range, double* _
     out[0] = a;
     out[1] = c;
   }
-}
-
-// Sharded runs: every rank owns the correspondences of its source range only.  When the caller asks for them
-// (get_source_correspondence) the ranges are merged through the all-reduce callback: each entry is encoded so that it is
-// non-zero on exactly one rank (index + 1, squared distance) and zero elsewhere — the sum is exact.
-__global__ void corr_pack_kernel(int n, int begin, int end, const int32_t* __restrict__ corr, const float* __restrict__ sqd,
-                                 double* __restrict__ out) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const bool mine = i >= begin && i < end;
-  out[i] = mine ? (double)(corr[i] + 1) : 0.0;
-  out[(size_t)n + i] = mine ? (double)sqd[i] : 0.0;
-}
-__global__ void corr_unpack_kernel(int n, const double* __restrict__ in, int32_t* __restrict__ corr, float* __restrict__ sqd) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  corr[i] = (int32_t)in[i] - 1;
-  sqd[i] = (float)in[(size_t)n + i];
 }
 
 // Mahalanobis + residual/Jacobian of ONE matched source point i <-> target point j (fgi:273-352): adds the point's 21 H
@@ -489,7 +459,7 @@ linearize_kernel(PoseD T, LinArgs a) {
     const int32_t j = a.corr[i];
     if (j >= 0) linearize_point(T, i, j, a.src_xyz, a.src_cov, a.tgt_xyz, a.tgt_cov, a.mahal, v);
   }
-  block_reduce_finalize<kRed>(v, a.partial, a.out, a.counter, a.host_out, a.host_seq, a.seq, a.comm, a.xseq);
+  block_reduce_finalize<kRed>(v, a.partial, a.counter, a.host_out, a.host_seq, a.seq, a.comm, a.xseq);
 }
 
 struct ErrArgs {
@@ -499,9 +469,8 @@ struct ErrArgs {
   const int32_t* corr;
   const double* mahal;
   double* partial;
-  double* out;  // [1]
   unsigned int* counter;
-  double* host_out;
+  double* host_out;        // mapped pinned [1]
   volatile unsigned long long* host_seq;
   unsigned long long seq;
   CommView comm;
@@ -516,7 +485,7 @@ error_kernel(PoseD T, ErrArgs a) {
     const int32_t j = a.corr[i];
     if (j >= 0) v[0] = error_point(T, i, j, a.src_xyz, a.tgt_xyz, a.mahal);
   }
-  block_reduce_finalize<1>(v, a.partial, a.out, a.counter, a.host_out, a.host_seq, a.seq, a.comm, a.xseq);
+  block_reduce_finalize<1>(v, a.partial, a.counter, a.host_out, a.host_seq, a.seq, a.comm, a.xseq);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -542,8 +511,8 @@ error_kernel(PoseD T, ErrArgs a) {
 constexpr int kLmBlock = 256;     // threads per block of align_lm_kernel
 constexpr int kLmChunk = 4;       // source points per warp visit
 constexpr int kLmSeg = 8;         // partial-sum segments per value in the cross-block reduction
-constexpr long long kLmPollBudget = 1ll << 27;
-constexpr int kLmPersistentMax = 65536;  // source points per rank up to which the persistent LM kernel is used  // barrier polls before giving up (seconds of wall time)
+constexpr long long kLmPollBudget = 1ll << 27;  // barrier polls before giving up (seconds of wall time)
+constexpr int kLmPersistentMax = 65536;  // source points per shard up to which the persistent LM kernel is used
 
 struct LmResult {  // lives in mapped pinned host memory; written by block 0
   double R[9], t[3];      // final pose x0
@@ -914,11 +883,6 @@ align_lm_kernel(LmArgs a) {
   }
 }
 
-__global__ void f64_to_f32_kernel(size_t n, const double* __restrict__ in, float* __restrict__ out) {
-  const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) out[i] = (float)in[i];
-}
-
 __global__ void identity_filter_kernel(int n, int32_t* f) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i < n) f[i] = i + 1;
@@ -975,18 +939,15 @@ struct gsicp_gicp {
   float final_transformation[16];
   double final_hessian[36];
   cudaStream_t stream = 0;
-  Scratch corr, sqd, mahal, partial, red_out, counter, staging_dev, nn_id, nn_d2;
+  Scratch corr, sqd, mahal, partial, red_out, counter, nn_id, nn_d2;
   int corr_n = 0;
-  double* h_red = nullptr;     // pinned [28]
   HostMailbox lin_box;         // linearize / error sums: [0, kRed) as doubles, [kRed] sequence word
   HostMailbox lm_box;          // LmResult of align_lm_kernel
   void* h_stage = nullptr;     // pinned staging for H2D conversions
   size_t h_stage_cap = 0;
-  int shard_count = 1, shard_index = 0;
-  gsicp_comm* comm = nullptr;    // in-library exchange over peer memory (gsicp_gicp_set_comm); replaces the callback
+  int shard_count = 1, shard_index = 0;  // the exchange group's world and rank (gsicp_gicp_set_comm)
+  gsicp_comm* comm = nullptr;    // in-library exchange over peer memory (gsicp_gicp_set_comm)
   bool src_partial = false;      // sharded covariances: this rank holds only its own source rotations / scales / covariances
-  gsicp_allreduce_fn reduce = nullptr;
-  void* reduce_user = nullptr;
   bool host_lm = false;          // gsicp_gicp_set_host_lm: host-driven LM loop (one launch + one spin-wait per phase)
   Scratch lm_partL, lm_partE, lm_barrier;
   int lm_max_blocks = 0;         // co-resident blocks of align_lm_kernel on this device
@@ -1237,12 +1198,10 @@ int ensure_lin_buffers(gsicp_gicp* h) {
   if (int e = h->sqd.ensure((size_t)(n + 1) * 4)) return e;
   if (int e = h->mahal.ensure((size_t)(n + 1) * 6 * sizeof(double))) return e;
   if (int e = h->partial.ensure((size_t)blocks * kRed * sizeof(double))) return e;
-  if (int e = h->red_out.ensure(kRed * sizeof(double))) return e;
   if (!h->counter.ptr) {
     if (int e = h->counter.ensure(sizeof(unsigned int))) return e;
     GSICP_CUDA(cudaMemsetAsync(h->counter.ptr, 0, sizeof(unsigned int), h->stream));
   }
-  if (!h->h_red) GSICP_CUDA(cudaMallocHost(&h->h_red, kRed * sizeof(double)));
   return h->lin_box.ensure((kRed + 1) * sizeof(unsigned long long));
 }
 
@@ -1321,25 +1280,11 @@ int comm_take_seq(gsicp_gicp* h, unsigned long long reserve, unsigned long long*
   return GSICP_OK;
 }
 
-// The n sums of a linearize / error launch into h->h_red.  Single-GPU and in-kernel-exchange runs read them from the mailbox
-// the kernel published into; a sharded run with the all-reduce callback sums red_out over the ranks and copies it back.
-int collect_sums(gsicp_gicp* h, int n, bool direct, unsigned long long seq) {
-  if (h->shard_count > 1 && h->reduce) {
-    const int rc = h->reduce(h->reduce_user, h->red_out.as<double>(), n, (void*)h->stream);
-    if (rc != 0) {
-      set_error("all-reduce callback failed (%d)", rc);
-      return GSICP_ECUDA;
-    }
-  }
-  if (direct) {
-    GSICP_CUDA(cudaGetLastError());
-    if (int e = h->lin_box.wait(kRed, seq, h->stream, "GICP reduction")) return e;
-    std::memcpy(h->h_red, h->lin_box.host, n * sizeof(double));
-  } else {
-    GSICP_CUDA(cudaMemcpyAsync(h->h_red, h->red_out.ptr, n * sizeof(double), cudaMemcpyDeviceToHost, h->stream));
-    GSICP_CUDA(cudaStreamSynchronize(h->stream));
-  }
-  return GSICP_OK;
+// Waits until the linearize / error launch numbered `seq` has published its sums into the mailbox; the caller then reads
+// them from lin_box.host.  In a sharded run the kernel's last block has already exchanged them: they are the global sums.
+int collect_sums(gsicp_gicp* h, unsigned long long seq) {
+  GSICP_CUDA(cudaGetLastError());
+  return h->lin_box.wait(kRed, seq, h->stream, "GICP reduction");
 }
 
 // fgi:296-352.  H may be null (error only).
@@ -1359,15 +1304,13 @@ int run_linearize(gsicp_gicp* h, const Iso& x, double H[6][6], double b[6], doub
   a.src_xyz = h->src.xyz.as<float>(); a.src_cov = h->src.cov.as<double>();
   a.tgt_xyz = h->tgt.xyz.as<float>(); a.tgt_cov = h->tgt.cov.as<double>();
   a.corr = h->corr.as<int32_t>(); a.sqd = h->sqd.as<float>(); a.mahal = h->mahal.as<double>();
-  a.partial = h->partial.as<double>(); a.out = h->red_out.as<double>(); a.counter = h->counter.as<unsigned int>();
-  const bool xchg = h->shard_count > 1 && h->comm;  // in-kernel exchange: the published sums are already global
-  const bool direct = h->shard_count <= 1 || xchg;   // publish straight into mapped host memory
-  a.host_out = direct ? (double*)h->lin_box.dev : nullptr;
-  a.host_seq = direct ? (volatile unsigned long long*)(h->lin_box.dev + kRed) : nullptr;
+  a.partial = h->partial.as<double>(); a.counter = h->counter.as<unsigned int>();
+  a.host_out = (double*)h->lin_box.dev;
+  a.host_seq = (volatile unsigned long long*)(h->lin_box.dev + kRed);
   a.seq = ++h->lin_box.seq;
   a.comm = CommView();
   a.xseq = 0;
-  if (xchg) {
+  if (h->shard_count > 1 && h->comm) {
     a.comm = h->comm->view();
     if (int e = comm_take_seq(h, 1, &a.xseq)) return e;
   }
@@ -1382,18 +1325,19 @@ int run_linearize(gsicp_gicp* h, const Iso& x, double H[6][6], double b[6], doub
                  a.src_xyz, a.corr, a.sqd);
   }
   GSICP_LAUNCH(linearize_kernel, blocks, kLinBlock, 0, h->stream, make_pose(x), a); }
-  if (int e = collect_sums(h, kRed, direct, a.seq)) return e;
+  if (int e = collect_sums(h, a.seq)) return e;
+  const double* sums = reinterpret_cast<const double*>(h->lin_box.host);
   if (H && b) {
     int o = 0;
     for (int r = 0; r < 6; r++)
       for (int c = r; c < 6; c++) {
-        H[r][c] = h->h_red[o];
-        H[c][r] = h->h_red[o];
+        H[r][c] = sums[o];
+        H[c][r] = sums[o];
         o++;
       }
-    for (int r = 0; r < 6; r++) b[r] = h->h_red[21 + r];
+    for (int r = 0; r < 6; r++) b[r] = sums[21 + r];
   }
-  *err = h->h_red[27];
+  *err = sums[27];
   return GSICP_OK;
 }
 
@@ -1405,15 +1349,13 @@ int run_error(gsicp_gicp* h, const Iso& x, double* err) {  // fgi:355-378
   a.begin = begin; a.end = end;
   a.src_xyz = h->src.xyz.as<float>(); a.tgt_xyz = h->tgt.xyz.as<float>();
   a.corr = h->corr.as<int32_t>(); a.mahal = h->mahal.as<double>();
-  a.partial = h->partial.as<double>(); a.out = h->red_out.as<double>(); a.counter = h->counter.as<unsigned int>();
-  const bool xchg = h->shard_count > 1 && h->comm;
-  const bool direct = h->shard_count <= 1 || xchg;
-  a.host_out = direct ? (double*)h->lin_box.dev : nullptr;
-  a.host_seq = direct ? (volatile unsigned long long*)(h->lin_box.dev + kRed) : nullptr;
+  a.partial = h->partial.as<double>(); a.counter = h->counter.as<unsigned int>();
+  a.host_out = (double*)h->lin_box.dev;
+  a.host_seq = (volatile unsigned long long*)(h->lin_box.dev + kRed);
   a.seq = ++h->lin_box.seq;
   a.comm = CommView();
   a.xseq = 0;
-  if (xchg) {
+  if (h->shard_count > 1 && h->comm) {
     a.comm = h->comm->view();
     if (int e = comm_take_seq(h, 1, &a.xseq)) return e;
   }
@@ -1421,8 +1363,8 @@ int run_error(gsicp_gicp* h, const Iso& x, double* err) {  // fgi:355-378
   if (blocks < 1) blocks = 1;
   { ProfScope ps(kProfError, h->stream);
   GSICP_LAUNCH(error_kernel, blocks, kLinBlock, 0, h->stream, make_pose(x), a); }
-  if (int e = collect_sums(h, 1, direct, a.seq)) return e;
-  *err = h->h_red[0];
+  if (int e = collect_sums(h, a.seq)) return e;
+  *err = reinterpret_cast<const double*>(h->lin_box.host)[0];
   return GSICP_OK;
 }
 
@@ -1594,11 +1536,10 @@ void gsicp_gicp_destroy(gsicp_gicp* h) {
     fr(c->grid.meta_buf); fr(c->grid.bbox_buf); fr(c->grid.cell_start); fr(c->grid.cursor); fr(c->grid.cell_of_pt);
     fr(c->grid.pts); fr(c->grid.cub_tmp);
   }
-  fr(h->corr); fr(h->sqd); fr(h->mahal); fr(h->partial); fr(h->red_out); fr(h->counter); fr(h->staging_dev); fr(h->nn_id); fr(h->nn_d2);
+  fr(h->corr); fr(h->sqd); fr(h->mahal); fr(h->partial); fr(h->red_out); fr(h->counter); fr(h->nn_id); fr(h->nn_d2);
   fr(h->lm_partL); fr(h->lm_partE); fr(h->lm_barrier);
   h->lm_box.release();
   h->lin_box.release();
-  if (h->h_red) cudaFreeHost(h->h_red);
   if (h->h_stage) cudaFreeHost(h->h_stage);
   delete h;
 }
@@ -1696,12 +1637,13 @@ int gsicp_gicp_align(gsicp_gicp* h, const float guess[16], float out[16]) {
   }
   h->lm_lambda = -1.0;
   int iters = 0;
-  int lb, le;
-  shard_range(h, h->src.n, lb, le);
   // The persistent kernel (one block per SM) wins where launch / wait latency dominates; above kLmPersistentMax points per
-  // rank the phases are throughput-bound and the full-occupancy kernels of the host-driven loop are faster
+  // shard the phases are throughput-bound and the full-occupancy kernels of the host-driven loop are faster
   // (in a sharded run their last block exchanges through the peers' segments as well: no host-side collective either way).
-  if (!h->host_lm && (h->shard_count <= 1 || h->comm) && (le - lb) <= kLmPersistentMax) {
+  // The two loops use exchange sequence numbers differently, so every rank of a group must take the same one: decide from
+  // the size of rank 0's shard (shard_range's ceil(n / shard_count)), which is the same on every rank.
+  const long long shard0 = ((long long)h->src.n + h->shard_count - 1) / h->shard_count;
+  if (!h->host_lm && shard0 <= kLmPersistentMax) {
     // device-resident LM loop: one persistent kernel, zero host round trips inside the loop
     if (h->lm_box.host) std::memset(reinterpret_cast<LmResult*>(h->lm_box.host)->H, 0, sizeof(LmResult::H));
     iters = run_align_device(h, x0);
@@ -1764,19 +1706,6 @@ int gsicp_gicp_get_source_correspondence(gsicp_gicp* h, int32_t* corr, float* sq
     GSICP_CUDA(cudaMemsetAsync(h->sqd.as<float>(), 0, (size_t)begin * 4, h->stream));
     if (end < h->src.n) GSICP_CUDA(cudaMemsetAsync(h->sqd.as<float>() + end, 0, (size_t)(h->src.n - end) * 4, h->stream));
     if (int e = comm_sum_merge<float>(h, h->sqd.as<float>(), (size_t)h->src.n)) return e;
-  } else if (h->shard_count > 1 && h->reduce) {  // merge the ranks' ranges (SURVEY §8e: gathered only when asked for)
-    const int n = h->src.n;
-    int begin, end;
-    shard_range(h, n, begin, end);
-    if (int e = h->staging_dev.ensure((size_t)n * 2 * sizeof(double))) return e;
-    double* buf = h->staging_dev.as<double>();
-    GSICP_LAUNCH(corr_pack_kernel, (n + 255) / 256, 256, 0, h->stream, n, begin, end, h->corr.as<int32_t>(), h->sqd.as<float>(), buf);
-    if (h->reduce(h->reduce_user, buf, 2 * n, (void*)h->stream) != 0) {
-      set_error("all-reduce callback failed");
-      return GSICP_ECUDA;
-    }
-    GSICP_LAUNCH(corr_unpack_kernel, (n + 255) / 256, 256, 0, h->stream, n, buf, h->corr.as<int32_t>(), h->sqd.as<float>());
-    GSICP_CUDA(cudaGetLastError());
   }
   GSICP_CUDA(cudaMemcpyAsync(corr, h->corr.ptr, (size_t)h->src.n * 4, cudaMemcpyDeviceToHost, h->stream));
   GSICP_CUDA(cudaMemcpyAsync(sq_dist, h->sqd.ptr, (size_t)h->src.n * 4, cudaMemcpyDeviceToHost, h->stream));
@@ -1853,14 +1782,6 @@ int gsicp_gicp_compute_error(gsicp_gicp* h, const double pose[16], double* err) 
   return run_error(h, x, err);
 }
 
-int gsicp_gicp_set_shard(gsicp_gicp* h, int count, int index, gsicp_allreduce_fn reduce, void* user) {
-  H_CHECK(h);
-  if (count < 1 || index < 0 || index >= count) return GSICP_EINVAL;
-  h->shard_count = count; h->shard_index = index; h->reduce = reduce; h->reduce_user = user;
-  h->corr_n = -1;
-  return GSICP_OK;
-}
-
 int gsicp_gicp_set_comm(gsicp_gicp* h, gsicp_comm* comm) {
   H_CHECK(h);
   if (comm && !comm->connected) {
@@ -1870,8 +1791,6 @@ int gsicp_gicp_set_comm(gsicp_gicp* h, gsicp_comm* comm) {
   h->comm = comm;
   h->shard_count = comm ? comm->world : 1;
   h->shard_index = comm ? comm->rank : 0;
-  h->reduce = nullptr;
-  h->reduce_user = nullptr;
   h->corr_n = -1;
   h->src.clear_cov();
   return GSICP_OK;
@@ -1889,9 +1808,9 @@ extern "C" int gsicp_test_preload_kernels(void) {
   const void* fns[] = {(const void*)knn_kernel<10>, (const void*)knn_kernel<20>, (const void*)knn_kernel<32>,
                        (const void*)covariance_kernel<10>, (const void*)covariance_kernel<20>, (const void*)covariance_kernel<32>,
                        (const void*)compact_xyz_kernel, (const void*)cov_from_qs_kernel, (const void*)correspond_kernel,
-                       (const void*)fitness_kernel, (const void*)corr_pack_kernel, (const void*)corr_unpack_kernel,
+                       (const void*)fitness_kernel,
                        (const void*)linearize_kernel, (const void*)error_kernel, (const void*)align_lm_kernel,
-                       (const void*)f64_to_f32_kernel, (const void*)identity_filter_kernel,
+                       (const void*)identity_filter_kernel,
                        (const void*)comm_stage_kernel<int32_t>, (const void*)comm_stage_kernel<float>, (const void*)comm_stage_kernel<double>,
                        (const void*)comm_stage_corr_kernel,
                        (const void*)comm_sum_kernel<int32_t>, (const void*)comm_sum_kernel<float>, (const void*)comm_sum_kernel<double>};

@@ -23,7 +23,6 @@
 #include "host_common.h"
 #include "raster_common.cuh"
 #include "comm.cuh"
-#include "scan.cuh"
 
 namespace gsicp {
 
@@ -666,37 +665,9 @@ extern int g_render_cull;
 int g_bwd_variant = [] { const char* e = getenv("GSICP_BWD_VARIANT"); return e ? atoi(e) : 0; }();
 
 // ---- multi-GPU: all-reduce of the render moments of the VISIBLE Gaussians (SURVEY §8e) ----
-// Every rank preprocesses all Gaussians, so the set {radii > 0} and its index order are identical on all ranks: the
-// moments of those V Gaussians are gathered into a dense [V][12] buffer, summed over the ranks by the caller's
-// collective (NCCL over NVLink) and scattered back; the per-Gaussian backward then runs replicated.  12*V floats
-// travel instead of the 14*P parameter gradients (33k vs 300k Gaussians in config C3).
-struct VisibleFlag {
-  const int32_t* radii;
-  __host__ __device__ uint32_t operator()(int i) const { return radii[i] > 0 ? 1u : 0u; }
-};
-
-__global__ void publish_visible_kernel(int P, const uint32_t* __restrict__ excl, const int32_t* __restrict__ radii,
-                                       volatile unsigned long long* host_map, unsigned long long seq) {
-  host_map[0] = (unsigned long long)(excl[P - 1] + (radii[P - 1] > 0 ? 1u : 0u));
-  __threadfence_system();
-  host_map[1] = seq;
-  __threadfence_system();
-}
-
-template <bool kGather>
-__global__ void moments_compact_kernel(int P, const int32_t* __restrict__ radii, const uint32_t* __restrict__ excl,
-                                       float* __restrict__ moments, float* __restrict__ dense) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= P || !(radii[i] > 0)) return;
-  float4* m = reinterpret_cast<float4*>(moments) + 3 * (size_t)i;
-  float4* d = reinterpret_cast<float4*>(dense) + 3 * (size_t)excl[i];
-#pragma unroll
-  for (int k = 0; k < 3; k++) {
-    if (kGather) d[k] = m[k];
-    else m[k] = d[k];
-  }
-}
-
+// Every rank preprocesses all Gaussians, so the set {radii > 0} and its index order are identical on all ranks; only the
+// moments of those Gaussians are summed over the ranks, and the per-Gaussian backward then runs replicated.
+//
 // Sharded run through the exchange layer (comm.cuh): every rank's render_backward accumulated the moments of ITS tiles in
 // its own segment.  The all-reduce over the ranks is two P2P passes over NVLink, both inside our kernels:
 //   reduce-scatter: rank r adds, in rank order, the world's rows of the visible Gaussians of ITS slice of the table
@@ -733,47 +704,13 @@ __global__ void moments_gather_slices_kernel(CommView c, int P, int slice, const
 }
 
 gsicp_comm* g_raster_comm = nullptr;  // set by gsicp_raster_set_comm; also read by the forward pass (raster_forward.cu)
+static std::mutex g_raster_comm_mu;   // serialises gsicp_raster_set_comm
 
 // Where this rank's render moments accumulate: the exchange segment in a sharded run, else the geometry buffer.
 float* raster_moment_accumulator(const gsicp_raster_args* args, float* geom_moments) {
   gsicp_comm* c = g_raster_comm;
   if (!c || c->world <= 1 || args->tile_shard_count <= 1) return geom_moments;
   return reinterpret_cast<float*>(c->local + kCommHeapOff);
-}
-
-struct BwdShared {
-  std::mutex mu;
-  gsicp_allreduce_f32_fn fn = nullptr;
-  void* user = nullptr;
-  Scratch excl, dense, cub_tmp;
-  HostMailbox box;  // [0] visible count V, [1] sequence word
-};
-static BwdShared g_bwd;
-
-static int allreduce_visible_moments(int P, const int32_t* d_radii, float* moments, cudaStream_t stream) {
-  std::lock_guard<std::mutex> lock(g_bwd.mu);
-  HostMailbox& box = g_bwd.box;
-  if (int e = box.ensure(2 * sizeof(unsigned long long))) return e;
-  if (int e = flag_exclusive_scan<uint32_t>(P, VisibleFlag{d_radii}, g_bwd.excl, g_bwd.cub_tmp, stream)) return e;
-  const unsigned long long seq = ++box.seq;
-  GSICP_LAUNCH(publish_visible_kernel, 1, 1, 0, stream, P, g_bwd.excl.as<uint32_t>(), d_radii,
-               (volatile unsigned long long*)box.dev, seq);
-  GSICP_CUDA(cudaGetLastError());
-  if (int e = box.wait(1, seq, stream, "visible Gaussian count")) return e;
-  const size_t V = (size_t)box.host[0];
-  if (V == 0) return GSICP_OK;
-  if (int e = g_bwd.dense.ensure(V * kG * sizeof(float))) return e;
-  GSICP_LAUNCH(moments_compact_kernel<true>, (P + 255) / 256, 256, 0, stream, P, d_radii, g_bwd.excl.as<uint32_t>(), moments,
-               g_bwd.dense.as<float>());
-  const int rc = g_bwd.fn(g_bwd.user, g_bwd.dense.as<float>(), V * kG, (void*)stream);
-  if (rc != 0) {
-    set_error("rasterizer all-reduce callback failed (%d)", rc);
-    return GSICP_ECUDA;
-  }
-  GSICP_LAUNCH(moments_compact_kernel<false>, (P + 255) / 256, 256, 0, stream, P, d_radii, g_bwd.excl.as<uint32_t>(), moments,
-               g_bwd.dense.as<float>());
-  GSICP_CUDA(cudaGetLastError());
-  return GSICP_OK;
 }
 
 }  // namespace gsicp
@@ -796,13 +733,6 @@ static int ensure_bwd_smem_attr() {
   return GSICP_OK;
 }
 
-extern "C" int gsicp_raster_set_allreduce(gsicp_allreduce_f32_fn fn, void* user) {
-  std::lock_guard<std::mutex> lock(g_bwd.mu);
-  g_bwd.fn = fn;
-  g_bwd.user = user;
-  return GSICP_OK;
-}
-
 // The render moments live in the geometry buffer the forward pass allocated (GeomState::moments, zeroed for the visible
 // Gaussians by preprocess): the backward needs no caller-provided work buffer any more.  Kept for ABI stability.
 extern "C" int gsicp_raster_set_comm(gsicp_comm* comm) {
@@ -810,7 +740,7 @@ extern "C" int gsicp_raster_set_comm(gsicp_comm* comm) {
     set_error("gsicp_raster_set_comm: the exchange group is not connected");
     return GSICP_ESTATE;
   }
-  std::lock_guard<std::mutex> lock(g_bwd.mu);
+  std::lock_guard<std::mutex> lock(g_raster_comm_mu);
   g_raster_comm = comm;
   return GSICP_OK;
 }
@@ -885,8 +815,6 @@ extern "C" int gsicp_raster_backward(const gsicp_raster_args* args, int num_rend
     GSICP_LAUNCH(moments_gather_slices_kernel, (P + 255) / 256, 256, 0, stream, comm->view(), P, slice, d_radii, red_off, geom.moments);
     xmom = work;
     work = geom.moments;
-  } else if (shard_count > 1 && g_bwd.fn) {
-    if (int e = allreduce_visible_moments(P, d_radii, work, stream)) return e;
   }
 
   BwdArgs ba;

@@ -265,19 +265,3 @@ class FastGICP:
     def set_host_lm(self, on):
         """Test / A-B hook: drive the LM loop from the host instead of the device-resident kernel (same results)."""
         check(lib.gsicp_gicp_set_host_lm(self._h, int(bool(on))))
-
-    def set_shard(self, count, index, reduce_cb=None):
-        """Shard the source points over `count` ranks; reduce_cb(device_ptr, count, stream) all-reduces in place."""
-        if reduce_cb is None:
-            self._cb = _lib.ALLREDUCE_FN()
-        else:
-            def _tramp(_user, ptr, cnt, stream):
-                try:
-                    reduce_cb(ptr, cnt, stream)
-                    return 0
-                except Exception as ex:  # never let an exception cross the C boundary
-                    print(f"all-reduce callback failed: {ex}", file=sys.stderr)
-                    return 1
-
-            self._cb = _lib.ALLREDUCE_FN(_tramp)
-        check(lib.gsicp_gicp_set_shard(self._h, int(count), int(index), self._cb, None))

@@ -26,30 +26,6 @@ def set_tile_shard(count, index):
     _tile_shard = (int(count), int(index))
 
 
-_allreduce_cb = None  # keeps the ctypes thunk alive
-
-
-def set_allreduce(fn):
-    """Multi-GPU: fn(device_ptr, count, stream) sums `count` float32 values in place over the ranks (or None to clear).
-    With tile sharding active, rasterize_gaussians_backward then returns the full (already summed) gradients."""
-    global _allreduce_cb
-    if fn is None:
-        _allreduce_cb = _lib.ALLREDUCE_F32_FN()
-    else:
-        def _tramp(_user, ptr, count, stream):
-            try:
-                fn(ptr, count, stream)
-                return 0
-            except Exception as ex:  # never let an exception cross the C boundary
-                import sys
-
-                print(f"rasterizer all-reduce callback failed: {ex}", file=sys.stderr)
-                return 1
-
-        _allreduce_cb = _lib.ALLREDUCE_F32_FN(_tramp)
-    check(lib.gsicp_raster_set_allreduce(_allreduce_cb, None))
-
-
 def set_comm(comm):
     """Multi-GPU: the library's own exchange group (gs_icp_slam_b200.sharding.ShardGroup) or None.  With tile sharding
     active, rasterize_gaussians_backward exchanges the render moments through the peers' device segments inside the call."""

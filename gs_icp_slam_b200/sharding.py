@@ -5,8 +5,9 @@
   moments of the ranks add up inside gsicp_raster_backward, so every rank ends with the complete parameter gradients.
 * GICP: source points are split into contiguous ranges (k-NN covariances and the LM loop); the 28 doubles of the normal
   equations (21 H + 6 b + error) are exchanged at every reduction point.
-`ShardGroup` wires both to the library's in-kernel exchange over peer memory (csrc/comm.cuh) and falls back to
-torch.distributed collectives reached through the library's callbacks; the helpers above it serve the fallback and the tests.
+`ShardGroup` wires both to the library's in-kernel exchange over peer memory (csrc/comm.cuh), which needs CUDA IPC
+between the ranks.  The module-level helpers partition pixels (tile_owner_mask, sharded_l1) and source points
+(source_range), and sum the gradients of parameters that live outside the library (allreduce_grads).
 """
 import torch
 
@@ -48,73 +49,21 @@ def allreduce_grads(params, group=None):
         off += n
 
 
-class DevicePtrArray:
-    """Zero-copy view of `count` float64 values at a raw device pointer (CUDA array interface), so the library's
-    reduction buffer can be handed to torch.distributed.all_reduce."""
-
-    def __init__(self, ptr, count, typestr="<f8"):
-        self.__cuda_array_interface__ = {"shape": (int(count),), "typestr": typestr, "data": (int(ptr), False), "version": 3}
-
-
-def _lib_stream(stream, device):
-    """torch view of the cudaStream_t the library passed to a collective callback (0 = the legacy default stream): the
-    collective must be ordered after the kernels on THAT stream and before the library's readback on it, not on torch's
-    current stream of the calling thread."""
-    if not stream or not torch.cuda.is_available():
-        return torch.cuda.default_stream(device) if torch.cuda.is_available() else None
-    return torch.cuda.ExternalStream(int(stream), device=device)
-
-
-def make_gicp_allreduce(device, group=None):
-    """Callback for FastGICP.set_shard: all-reduces the library's fp64 buffer in place over `group`."""
-    import torch.distributed as dist
-
-    def cb(ptr, count, stream):
-        t = torch.as_tensor(DevicePtrArray(ptr, count), device=device)
-        with torch.cuda.stream(_lib_stream(stream, device)):  # the stream the library launched its kernels on
-            dist.all_reduce(t, group=group)
-
-    return cb
-
-
-def make_raster_allreduce(device, group=None):
-    """Callback for rasterizer.set_allreduce: sums the dense [V][12] fp32 moment buffer over `group` (NCCL)."""
-    import torch.distributed as dist
-
-    def cb(ptr, count, stream):
-        t = torch.as_tensor(DevicePtrArray(ptr, count, "<f4"), device=device)
-        with torch.cuda.stream(_lib_stream(stream, device)):
-            dist.all_reduce(t, group=group)
-
-    return cb
-
-
 class ShardGroup:
     """One rank's membership of a sharded run: wires the rasterizer (tile shards + render-moment exchange) and FastGICP
     objects (source-point shards for the k-NN covariances and the LM loop + normal-equation exchange) to the exchange layer.
 
-    Preferred transport ("p2p"): the library's own exchange group (csrc/comm.cuh) — every rank allocates a symmetric
-    device segment, the 64-byte CUDA IPC handles travel once through torch.distributed.all_gather_object, and from then on
-    the kernels exchange through the peers' segments over NVLink with device-side flags: no host-launched collective, no
-    Python in the loop.  Fallback ("nccl-callback", used when CUDA IPC is unavailable): torch.distributed all-reduces
-    reached through the library's callbacks, ordered on the library's stream."""
+    The exchange group is the library's own (csrc/comm.cuh): every rank allocates a symmetric device segment, the 64-byte
+    CUDA IPC handles travel once through torch.distributed.all_gather_object, and from then on the kernels exchange through
+    the peers' segments over NVLink with device-side flags: no host-launched collective, no Python in the loop.  The
+    constructor is collective; it raises on every rank when the group cannot be set up on all of them."""
 
-    def __init__(self, device, world, rank, group=None, heap_bytes=256 << 20, transport="auto"):
+    def __init__(self, device, world, rank, group=None, heap_bytes=256 << 20):
         self.device, self.world, self.rank, self.group = device, world, rank, group
         self._gicp = []
         self._raster = False
         self._comm = None
-        self.transport = "nccl-callback"
-        if transport in ("auto", "p2p") and world > 1:
-            try:
-                self._connect(heap_bytes)
-                self.transport = "p2p"
-            except Exception as ex:  # CUDA IPC not permitted in this environment
-                if transport == "p2p":
-                    raise
-                import sys
-
-                print(f"gs_icp_slam_b200.sharding: peer-memory exchange unavailable ({ex}); using the NCCL callbacks", file=sys.stderr)
+        self._connect(heap_bytes)
 
     def _connect(self, heap_bytes):
         import ctypes as C
@@ -145,47 +94,22 @@ class ShardGroup:
                 raise RuntimeError("exchange group could not be set up on every rank: " + (why or "a peer failed"))
         self._comm = comm
 
-    def _allreduce(self, typestr):
-        import torch.distributed as dist
-
-        dev, group = self.device, self.group
-
-        def cb(ptr, count, stream):
-            t = torch.as_tensor(DevicePtrArray(ptr, count, typestr), device=dev)
-            with torch.cuda.stream(_lib_stream(stream, dev)):  # after the kernels on the library's stream, before its readback
-                dist.all_reduce(t, group=group)
-
-        return cb
-
     def attach_rasterizer(self):
         from . import rasterizer
 
         rasterizer.set_tile_shard(self.world, self.rank)
-        if self._comm is not None:
-            rasterizer.set_comm(self._comm)
-        else:
-            rasterizer.set_allreduce(self._allreduce("<f4"))
+        rasterizer.set_comm(self._comm)
         self._raster = True
 
     def attach_gicp(self, reg):
-        if self._comm is not None:
-            reg.set_comm(self._comm)
-        else:
-            reg.set_shard(self.world, self.rank, self._allreduce("<f8"))
+        reg.set_comm(self._comm)
         self._gicp.append(reg)
-
-    def describe(self):
-        if self.transport == "p2p":
-            return ("in-kernel exchange through the peers' device segments (CUDA IPC over NVLink, device-side sequence flags): "
-                    "28-double normal equations inside the LM kernels, [visible][12] render moments inside the rasterizer's backward")
-        return "NCCL all-reduce (torch.distributed) of the 28-double normal equations / the [V][12] render moments on the library's stream"
 
     def close(self):
         if self._raster:
             from . import rasterizer
 
             rasterizer.set_tile_shard(1, 0)
-            rasterizer.set_allreduce(None)
             rasterizer.set_comm(None)
             self._raster = False
         for reg in self._gicp:

@@ -102,11 +102,9 @@ int gsicp_raster_forward(const gsicp_raster_args* args,
  * buffer of the forward pass: d_work is ignored (may be NULL) and gsicp_raster_backward_work_bytes() returns 0; both
  * are kept so that round-1 callers keep linking. */
 size_t gsicp_raster_backward_work_bytes(int P);
-/* Multi-GPU (tile-sharded rendering, SURVEY §8e): when set and tile_shard_count > 1, gsicp_raster_backward sums the 12
- * render moments of the visible Gaussians over the ranks through this callback (in place, fp32, on `stream`) between
- * the render-backward and the per-Gaussian-backward kernels; every rank then returns the FULL parameter gradients. */
-typedef int (*gsicp_allreduce_f32_fn)(void* user, float* d_buf, size_t count, void* stream);
-int gsicp_raster_set_allreduce(gsicp_allreduce_f32_fn fn, void* user);
+/* Multi-GPU (tile-sharded rendering, SURVEY §8e): with an exchange group set (gsicp_raster_set_comm) and
+ * tile_shard_count > 1, the 12 render moments of the visible Gaussians are summed over the ranks between the
+ * render-backward and the per-Gaussian-backward kernels; every rank then returns the FULL parameter gradients. */
 int gsicp_raster_backward(const gsicp_raster_args* args, int num_rendered,
                           const int32_t* d_radii,
                           const void* d_geom, const void* d_binning, const void* d_image,
@@ -206,7 +204,7 @@ int gsicp_gicp_get_source_rotationsq(gsicp_gicp*, float* out);
 int gsicp_gicp_get_target_rotationsq(gsicp_gicp*, float* out);
 int gsicp_gicp_get_source_scales(gsicp_gicp*, float* out);
 int gsicp_gicp_get_target_scales(gsicp_gicp*, float* out);
-/* main.cpp:230-233.  Sharded handles merge the ranks' ranges through the all-reduce callback first (collective call). */
+/* main.cpp:230-233.  Sharded handles merge the ranks' ranges through the exchange group first (collective call). */
 int gsicp_gicp_get_source_correspondence(gsicp_gicp*, int32_t* corr, float* sq_dist);
 /* Test/diagnostic access: regularised 3x3 covariances as 9 doubles per point (row-major). */
 int gsicp_gicp_get_source_covariances(gsicp_gicp*, double* out);
@@ -216,13 +214,6 @@ int gsicp_gicp_get_target_covariances(gsicp_gicp*, double* out);
  * b[6]; returns error through *err.  Used by the parity tests and by bench.py's roofline leg. */
 int gsicp_gicp_linearize(gsicp_gicp*, const double pose[16], double H[36], double b[6], double* err);
 int gsicp_gicp_compute_error(gsicp_gicp*, const double pose[16], double* err);
-
-/* Multi-GPU (SURVEY §8e): shard the SOURCE points [shard_index::shard_count) and all-reduce the
- * 28 doubles (21 H + 6 b + err) through the callback (torch.distributed / NCCL on the host side,
- * or ncclAllReduce inside the library when comm != NULL).  reduce(user, d_buf28, stream). */
-typedef int (*gsicp_allreduce_fn)(void* user, double* d_buf, int count, void* stream);
-int gsicp_gicp_set_shard(gsicp_gicp*, int shard_count, int shard_index,
-                         gsicp_allreduce_fn reduce, void* user);
 
 /* ---- Multi-GPU exchange group (one process per GPU; replaces the survey sketch's gsicp_gicp_comm_init(ncclComm_t)) ----
  * Each rank allocates a symmetric device segment and exports it as a 64-byte CUDA IPC handle; after the application
@@ -247,13 +238,18 @@ int gsicp_comm_connect_local(gsicp_comm*, int world, int rank, gsicp_comm* const
 int gsicp_comm_world(const gsicp_comm*);
 int gsicp_comm_rank(const gsicp_comm*);
 int gsicp_comm_barrier(gsicp_comm*, void* stream);   /* stream-ordered barrier over the group */
-int gsicp_gicp_set_comm(gsicp_gicp*, gsicp_comm*);    /* NULL: back to single-GPU */
-int gsicp_raster_set_comm(gsicp_comm*);               /* NULL: back to single-GPU; also sets the tile shard (count, index) */
+/* The handle shards its source points over the group: shard count and index are the group's world and rank.
+ * NULL: back to single-GPU. */
+int gsicp_gicp_set_comm(gsicp_gicp*, gsicp_comm*);
+/* Stores the group only; the tile shard still comes from gsicp_raster_args (tile_shard_count, tile_shard_index).
+ * NULL: back to single-GPU. */
+int gsicp_raster_set_comm(gsicp_comm*);
 
 /* Stream on which the handle's kernels run (default: legacy default stream 0). */
 int gsicp_gicp_set_stream(gsicp_gicp*, void* stream);
 /* Test / A-B hook: 1 = drive the LM loop from the host (one launch + one wait per linearize / compute_error), 0 (default) =
- * the device-resident loop (one persistent kernel per align, lsq_registration_impl.hpp:53-173 on the GPU).  Same results. */
+ * the device-resident loop (one persistent kernel per align, lsq_registration_impl.hpp:53-173 on the GPU).  Same results.
+ * In a sharded run the setting must be the same on every rank of the group: the two loops exchange differently. */
 int gsicp_gicp_set_host_lm(gsicp_gicp* h, int on);
 
 /* ---- fused mapping loss (SURVEY.md §8f row N2; the caller side of the rasterizer) ----------------------------------

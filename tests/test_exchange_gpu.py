@@ -60,19 +60,25 @@ def _run_ranks(world, fn):
     return out
 
 
-def _two_ranks_match_single(host_lm):
+def _two_ranks_match_single(host_lm, n_trackable=None):
     import gs_icp_slam_b200  # noqa: F401  (registers the drop-in module names)
     import pygicp
     from gs_icp_slam_b200._lib import lib
 
-    tgt, src, T = S.gicp_pair(30000, 20000, 60, 61)
+    if n_trackable is None:
+        tgt, src, T = S.gicp_pair(30000, 20000, 60, 61)
+        trk = np.arange(0, len(src), 3)  # a trackable subset: covariance slots differ from point indices
+        corr_dist = 0.05
+    else:
+        tgt, src, T = S.gicp_pair(150000, 150000, 62, 63, 0.001, scale=2.0)
+        trk = np.arange(n_trackable)
+        corr_dist = 0.1
     filt_t = np.arange(1, len(tgt) + 1, dtype=np.int32)
-    trk = np.arange(0, len(src), 3)  # a trackable subset: covariance slots differ from point indices
     filt_s = S.trackable_filter(len(src), trk)
 
     def make():
         r = pygicp.FastGICP()
-        r.set_max_correspondence_distance(0.05)
+        r.set_max_correspondence_distance(corr_dist)
         r.set_max_knn_distance(99999)
         r.set_host_lm(host_lm)
         return r
@@ -125,12 +131,15 @@ def _two_ranks_match_single(host_lm):
 
 def test_two_ranks_on_one_gpu_match_single(cuda):
     """Both LM drivers (persistent kernel with in-kernel exchange; host-driven kernels with the exchange in the last block) in
-    ONE child process (a hang there cannot take the pytest process and its CUDA context with it)."""
+    ONE child process (a hang there cannot take the pytest process and its CUDA context with it).  The third case has
+    131 073 trackable source points: rank 0's shard (65 537) lies above kLmPersistentMax and rank 1's (65 536) does not,
+    and both ranks must still run the same LM driver."""
     env = dict(os.environ)
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     env["PYTHONPATH"] = root + os.pathsep + env.get("PYTHONPATH", "")
     p = subprocess.run([sys.executable, os.path.abspath(__file__)], env=env, cwd=root, capture_output=True, text=True, timeout=150)
-    assert p.returncode == 0 and "EXCHANGE-OK False" in p.stdout and "EXCHANGE-OK True" in p.stdout, p.stdout[-2000:] + p.stderr[-4000:]
+    ok = all(f"EXCHANGE-OK {case}" in p.stdout for case in ("False", "True", "131073"))
+    assert p.returncode == 0 and ok, p.stdout[-2000:] + p.stderr[-4000:]
 
 
 if __name__ == "__main__":
@@ -146,3 +155,5 @@ if __name__ == "__main__":
     for host_lm in (False, True):
         _two_ranks_match_single(host_lm)
         print("EXCHANGE-OK", host_lm, "at %.1f s" % (time.time() - t0), flush=True)
+    _two_ranks_match_single(False, n_trackable=131073)
+    print("EXCHANGE-OK 131073 at %.1f s" % (time.time() - t0), flush=True)

@@ -1,6 +1,6 @@
 """Multi-GPU parity (needs >= 2 GPUs; run with `gpurun --gpus 2 -- python -m pytest tests/test_multigpu_gpu.py -m gpu`):
-tile-sharded rasterizer + point-sharded GICP must reproduce the single-GPU results, through both transports: the
-library's in-kernel exchange over peer memory (CUDA IPC / NVLink) and the NCCL-callback fallback."""
+tile-sharded rasterizer + point-sharded GICP must reproduce the single-GPU results through the library's in-kernel
+exchange over peer memory (CUDA IPC / NVLink)."""
 import os
 import subprocess
 import sys
@@ -43,7 +43,7 @@ def render(grp):
             ((color - gt).abs().mean() + 0.1 * (depth - gt[:1]).abs().mean()).backward()
             img = color.detach()
         out.append((img, {k: t[k].grad.clone() for k in t}, radii))
-    if shard: R.set_tile_shard(1, 0); R.set_allreduce(None); R.set_comm(None)
+    if shard: R.set_tile_shard(1, 0); R.set_comm(None)
     return out
 
 tgt, src, T = S.gicp_pair(30000, 20000, 60, 61)
@@ -59,26 +59,23 @@ def align(grp, host_lm, clouds=(tgt, src), corr_dist=0.05):
 img1, g1, r1 = render(None)[0]
 p1 = align(None, False)
 pb = align(None, False, (big_t, big_s), 0.1)
-for transport in ("p2p", "nccl-callback"):
-    grp = sharding.ShardGroup(dev, world, rank, transport="auto" if transport == "p2p" else "none")
-    if transport == "p2p":
-        assert grp.transport == "p2p", "peer-memory exchange could not be set up"
-    for imgN, gN, rN in render(grp):
-        assert torch.equal(r1, rN)
-        assert torch.equal(img1, imgN), "sharded image differs"
-        for k in g1:
-            err = (g1[k] - gN[k]).abs().max() / (g1[k].abs().max() + 1e-30)
-            assert err < 2e-4, (transport, k, float(err))
-    for host_lm in ((False, True) if transport == "p2p" else (True,)):
-        pN = align(grp, host_lm)
-        assert p1[1] == pN[1] and np.abs(p1[0] - pN[0]).max() <= 1e-6, (transport, host_lm, p1[1], pN[1], np.abs(p1[0] - pN[0]).max())
-        assert np.array_equal(p1[2][0], pN[2][0]) and np.array_equal(p1[2][1], pN[2][1]), "sharded correspondences differ after the merge"
-        assert np.array_equal(p1[3], pN[3]) and np.array_equal(p1[4], pN[4]), "sharded rotations / scales differ after the merge"
-    if transport == "p2p":   # above kLmPersistentMax points per rank: the full-occupancy kernels with in-kernel exchange
-        pN = align(grp, False, (big_t, big_s), 0.1)
-        assert pb[1] == pN[1] and np.abs(pb[0] - pN[0]).max() <= 1e-6
-        assert np.array_equal(pb[2][0], pN[2][0])
-    grp.close()
+grp = sharding.ShardGroup(dev, world, rank)
+for imgN, gN, rN in render(grp):
+    assert torch.equal(r1, rN)
+    assert torch.equal(img1, imgN), "sharded image differs"
+    for k in g1:
+        err = (g1[k] - gN[k]).abs().max() / (g1[k].abs().max() + 1e-30)
+        assert err < 2e-4, (k, float(err))
+for host_lm in (False, True):
+    pN = align(grp, host_lm)
+    assert p1[1] == pN[1] and np.abs(p1[0] - pN[0]).max() <= 1e-6, (host_lm, p1[1], pN[1], np.abs(p1[0] - pN[0]).max())
+    assert np.array_equal(p1[2][0], pN[2][0]) and np.array_equal(p1[2][1], pN[2][1]), "sharded correspondences differ after the merge"
+    assert np.array_equal(p1[3], pN[3]) and np.array_equal(p1[4], pN[4]), "sharded rotations / scales differ after the merge"
+# above kLmPersistentMax points per rank: the full-occupancy kernels with in-kernel exchange
+pN = align(grp, False, (big_t, big_s), 0.1)
+assert pb[1] == pN[1] and np.abs(pb[0] - pN[0]).max() <= 1e-6
+assert np.array_equal(pb[2][0], pN[2][0])
+grp.close()
 dist.barrier(); dist.destroy_process_group()
 if rank == 0: print("MULTIGPU_OK")
 '''

@@ -36,7 +36,7 @@ def _worker(rank, world, port, out):
         loss = sharding.sharded_l1(pred * w + b[:3, None, None], target, mask, pred.numel())
         loss.backward()
         sharding.allreduce_grads([w, b])
-        # normal equations: rank partial sums -> all-reduce (what the GICP callback does on the device buffer)
+        # normal equations: rank partial sums -> all-reduce (what the GICP kernels' in-kernel exchange computes)
         rows = torch.arange(100, dtype=torch.float64)[:, None] * torch.ones(28, dtype=torch.float64)
         lo, hi = sharding.source_range(100, world, rank)
         part = rows[lo:hi].sum(0)

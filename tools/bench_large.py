@@ -193,7 +193,7 @@ def main(args, rank, local_rank, world):
                "gpu_launches": int(launches),
                "config": {"workload": workload, "l2": "256 MiB write between steps, excluded from the per-step CUDA-event time"},
                "parallelism": "single GPU" if world == 1 else (f"{world} GPUs: " + ("screen tiles" if args.config == "c4" else "source points") +
-                                                                " sharded, " + (group.describe() if group else "")),
+                                                                " sharded, in-kernel exchange over peer memory"),
                "ms_p50_max": [float(np.median(ts)), float(np.max(ts))], "kernels": kern,
                "e2e": {"value": K / (t_ms * 1e-3), "unit": unit, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 64,
                        "note": "the public API call is what is timed; inputs are device tensors of the caller (the mapper's "
